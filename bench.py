@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- decoded channel-samples/s of the B200 Vorbis decode path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE config 4 -- 4,096 concurrent streams per GPU replicated /
@@ -142,6 +142,31 @@ def pinned_array(lib, nfloats):
         raise MemoryError("vpz_host_alloc(%d floats)" % nfloats)
     arr = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_float)), shape=(int(nfloats),))
     return arr, p
+
+
+def dump_outputs(batch, n_runs, out_dir, window=1024, budget_bytes=48 << 20):
+    """Writes what a caller of the timed path receives -- the fp32 PCM of every run of the batch as the last
+    decode left it -- so that two builds can be compared output for output.  All of it is ~8 GB per GPU, so:
+      pcm_windows.npy  float32: a window of `window` floats (fewer when `budget_bytes` or the run is smaller) of
+                       every run, at a seeded offset aligned to whole samples, the windows back to back;
+      run_samples.npy  float64: samples per channel of every run;
+      run_sums.npy     float64: the sum of every run's PCM, which every decoded value enters."""
+    os.makedirs(out_dir, exist_ok=True)
+    window = max(1, min(window, budget_bytes // (4 * max(n_runs, 1))))
+    rng = np.random.default_rng(0x5EED0004)
+    windows, samples, sums = [], np.zeros(n_runs), np.zeros(n_runs)
+    for run in range(n_runs):
+        pcm = batch.read_run(run)
+        flat = pcm.reshape(-1)
+        w = min(window, flat.size)
+        start = int(rng.integers(0, flat.size - w + 1))
+        start -= start % pcm.shape[1]
+        windows.append(flat[start:start + w])
+        samples[run] = pcm.shape[0]
+        sums[run] = flat.sum(dtype=np.float64)
+    np.save(os.path.join(out_dir, "pcm_windows.npy"), np.concatenate(windows).astype(np.float32))
+    np.save(os.path.join(out_dir, "run_samples.npy"), samples)
+    np.save(os.path.join(out_dir, "run_sums.npy"), sums)
 
 
 def run_reference(args, rank, world):
@@ -328,14 +353,13 @@ def run_config3(args, ctx, rank, world, barrier, max_over_ranks, sum_over_ranks,
     samples_rank = batch.total_floats
     clocks = ClockSampler(local_rank)
     clocks.start()
-    # one step is ~0.3 ms: warm up for ~0.4 s (also lets the clock sampler collect samples under load)
-    warm = max(args.warmup, 1500)
+    warm = args.warmup
     for _ in range(warm):
         batch.decode(clip=True, sync=False)
     batch.sync()
     barrier()
     launches0 = lib.vpz_ctx_kernel_launches(ctx._h)
-    steps = max(args.steps, 200)
+    steps = args.steps
     lib.vpz_ctx_mark(ctx._h, 0)
     for _ in range(steps):
         batch.decode(clip=True, sync=False)
@@ -470,8 +494,10 @@ def run_config5(args, ctx, rank, world, barrier, max_over_ranks, sum_over_ranks,
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    # one config3 step is ~0.3 ms: alone it defaults to 200 timed steps after ~0.4 s of warm-up (which also lets the
+    # clock sampler collect samples under load); the config3 sub-object of the default line uses the line's counts
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 5; 200 for --workload config3)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 3; 1500 for --workload config3)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--streams", type=int, default=4096, help="streams per GPU (weak) / in total (strong)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"])
@@ -485,10 +511,20 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-sub", action="store_true", help="skip the config3 / config5 sub-objects of the default line")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="config4 only: after the timed steps, write a fixed sample of the PCM the last of them decoded "
+                         "on rank 0 as DIR/*.npy (see dump_outputs)")
     ap.add_argument("--l1-bits", type=int, default=0, help=argparse.SUPPRESS)  # tuning: first-level Huffman table width
     ap.add_argument("--set", action="append", default=[], metavar="KEY=VALUE", help=argparse.SUPPRESS)  # any vpz_ctx_set tunable
     ap.add_argument("--lib", default=None, help=argparse.SUPPRESS)  # dry-run the script logic on the emulated test build
     args = ap.parse_args()
+    c3 = args.impl == "ours" and args.workload == "config3"
+    if args.steps is None:
+        args.steps = 200 if c3 else 5
+    if args.warmup is None:
+        args.warmup = 1500 if c3 else 3
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "config4"):
+        ap.error("--dump-outputs covers the default workload (--impl ours --workload config4)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -591,15 +627,16 @@ def main():
     batch = Batch(ctx)
     t_plan = time.perf_counter()
     n_pk = [f["n"] for f in per_file]
+    n_runs = 0
     for i in range(n_streams):
         g = first_stream + i
         fi, k = stream_file_and_start(g, len(files), n_pk)
         f = per_file[fi]
         # replica r starts at audio packet (7 r) mod count; the packets before it form a second run,
         # so every packet of the file is decoded once per replica (each run re-seeds its overlap)
-        batch.add_run_raw(f["setup"], f["blob"], np.ascontiguousarray(f["offs"][k:]))
+        n_runs = batch.add_run_raw(f["setup"], f["blob"], np.ascontiguousarray(f["offs"][k:])) + 1
         if k > 0:
-            batch.add_run_raw(f["setup"], f["blob"], np.ascontiguousarray(f["offs"][:k + 2]))
+            n_runs = batch.add_run_raw(f["setup"], f["blob"], np.ascontiguousarray(f["offs"][:k + 2])) + 1
     t_plan = time.perf_counter() - t_plan
     batch.upload()
     samples_rank = batch.total_floats          # one channel-sample = one fp32 PCM value
@@ -638,6 +675,11 @@ def main():
         k1b.append(a2)
         k3.append(b)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        # after the sampler stopped: `clocks` covers the decode steps, not the ~8 GB of copies the dump reads
+        t_dump = time.perf_counter()
+        dump_outputs(batch, n_runs, args.dump_outputs)
+        print("dump_outputs: %d runs in %.1f s" % (n_runs, time.perf_counter() - t_dump), file=sys.stderr)
     k1a_ms, k1b_ms, k3_ms = float(np.mean(k1a)), float(np.mean(k1b)), float(np.mean(k3))
     peak, peak_src = measured_peak()
     # algorithmic bytes per launch (DESIGN.md): K1a reads the packet bytes and writes the symbol

@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Generates tests/golden/ffmpeg_pin.npz: 16-bit PCM of the four TestFiles decoded by an INDEPENDENT
+"""Generates tests/golden/ffmpeg_pin_<name>.npz: 16-bit PCM of the four TestFiles decoded by an INDEPENDENT
 native Vorbis decoder (FFmpeg's `vorbis` decoder inside the libavcodec that ships in the
 opencv-python-headless wheel of this image), driven through ctypes.
 
@@ -9,7 +9,11 @@ nor libvorbisfile exists here, so the same convention is applied with a differen
 decoder.  The packets fed to FFmpeg come from a minimal Ogg page splitter in THIS file (no oracle
 code involved), so the pin is independent of the oracle's container layer as well.
 
-The generated file is committed; tests never need libavcodec or this script at run time.
+The generated files are committed; tests never need libavcodec or this script at run time.  Each holds
+the whole decode of one file as wrapping int16 second differences along time, split into a low-byte and a
+high-byte plane (`encode`): these deflate far better than the PCM itself and keep every file under 1 MB;
+two wrapping cumulative sums restore the PCM exactly.
+
 Layout knowledge used (FFmpeg 8 / lavc 62 public structs): AVPacket.data @24, .size @32;
 AVFrame.extended_data @96, .nb_samples @112, .format @116; AVCodecParameters.codec_type @0,
 .codec_id @4, .extradata @16, .extradata_size @24.
@@ -25,6 +29,15 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 FILES = ["1test", "2test", "3test", "issue6test"]
+
+
+def encode(q):
+    """q [frames, channels] int16 -> {"lo", "hi"}: the byte planes of its second differences, [channels, frames]."""
+    d = np.ascontiguousarray(q.T)
+    for _ in range(2):
+        d = np.diff(d, axis=1, prepend=np.int16(0)).astype(np.int16)
+    u = d.view(np.uint16)
+    return {"lo": (u & 0xFF).astype(np.uint8), "hi": (u >> 8).astype(np.uint8)}
 
 
 def ogg_packets(data):
@@ -75,7 +88,6 @@ def main():
     print("lavc version %x" % avc.avcodec_version())
     codec = avc.avcodec_find_decoder_by_name(b"vorbis")
     assert codec, "no native vorbis decoder in this libavcodec"
-    out = {}
     for name in FILES:
         data = open(os.path.join(ROOT, "tests", "data", name + ".ogg"), "rb").read()
         pk = ogg_packets(data)
@@ -127,9 +139,8 @@ def main():
         pcm = np.concatenate(chunks)
         q = np.clip((pcm * np.float32(32768.0)).astype(np.int64), -32768, 32767).astype(np.int16)
         print(name, pcm.shape, "rms %.5f" % float(np.sqrt((pcm.astype(np.float64) ** 2).mean())))
-        out[name] = q
-    np.savez_compressed(os.path.join(HERE, "ffmpeg_pin.npz"), **out)
-    print("wrote ffmpeg_pin.npz")
+        np.savez_compressed(os.path.join(HERE, "ffmpeg_pin_%s.npz" % name), **encode(q))
+        print("wrote ffmpeg_pin_%s.npz" % name)
 
 
 if __name__ == "__main__":

@@ -5,7 +5,9 @@ cpu_baseline / --impl reference legs.  The product package never imports this.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -358,19 +360,23 @@ _bench_libs = {}
 def bench_lib(native=False):
     """The oracle library used for TIMING: the portable -O2 build, or (native=True) the same sources built
     -O3 -march=native on THIS machine (oracle/Makefile `native`; rebuilt on every call site's first use so a
-    binary tuned for another CPU is never run).  None when that build is not possible here."""
+    binary tuned for another CPU is never run).  The native build goes to a temporary directory, removed once
+    the library is loaded, so the source tree may be read-only.  None when that build is not possible here."""
     key = bool(native)
     if key in _bench_libs:
         return _bench_libs[key]
     if not native:
         L = lib()
     else:
+        tmp = tempfile.mkdtemp(prefix="vpz_oracle_native_")
         try:
-            subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "-B", "native"], stdout=subprocess.DEVNULL,
-                                  stderr=subprocess.DEVNULL)
-            L = C.CDLL(os.path.join(ORACLE_DIR, "build_native", "libvorbis_oracle.so"))
+            subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "-B", "native", "NATIVE_DIR=" + tmp],
+                                  stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            L = C.CDLL(os.path.join(tmp, "libvorbis_oracle.so"))
         except Exception:
             L = None
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
     if L is not None:
         L.vo_bench_decode.restype = C.c_int64
         L.vo_bench_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double)]

@@ -2,7 +2,7 @@
 
 The reference is C# and ships no golden vectors for this path; no .NET runtime exists here.  The
 oracle is therefore pinned by (1) an INDEPENDENT native decoder (FFmpeg's vorbis decoder, fixture
-tests/golden/ffmpeg_pin.npz made by make_ffmpeg_pin.py) under the reference's own test convention
+tests/golden/ffmpeg_pin_<name>.npz made by make_ffmpeg_pin.py) under the reference's own test convention
 (NVorbis.Tests/AssetTest.cs:131-194: 16-bit PCM, |diff| <= 2 LSB, here even <= 1), (2) closed forms
 and invariants that do not depend on any decoder, (3) the workload counts SURVEY.md measured with a
 separate symbol-level walker, (4) regression digests of its own output (oracle_golden.json)."""
@@ -23,9 +23,18 @@ def q16(x):
     return np.clip((x * np.float32(32768.0)).astype(np.int64), -32768, 32767)
 
 
+def ffmpeg_pin(name):
+    """FFmpeg's 16-bit PCM of `name`, [frames, channels] (stored by make_ffmpeg_pin.encode)."""
+    z = np.load(os.path.join(GOLDEN, "ffmpeg_pin_%s.npz" % name))
+    d = (z["lo"].astype(np.uint16) | (z["hi"].astype(np.uint16) << 8)).view(np.int16)
+    for _ in range(2):
+        d = np.cumsum(d, axis=1, dtype=np.int16)
+    return d.T
+
+
 @pytest.mark.parametrize("name", FILES)
 def test_oracle_vs_independent_decoder(name):
-    pin = np.load(os.path.join(GOLDEN, "ffmpeg_pin.npz"))[name].astype(np.int64)
+    pin = ffmpeg_pin(name).astype(np.int64)
     s = ob.OracleStream(load_file(name))
     s.set_clip(False)
     pcm, _, _ = s.decode_all()
