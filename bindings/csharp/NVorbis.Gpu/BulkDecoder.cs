@@ -1,5 +1,5 @@
 // Bulk calls: many container images per call, pipelined on the GPU (vpz_decode_files / _s16 / vpz_decode_excerpts /
-// vpz_scan_pages).  These have no counterpart in the reference's API; they are what a server decoding thousands of
+// their _device forms / vpz_scan_pages).  These have no counterpart in the reference's API; they are what a server decoding thousands of
 // streams calls instead of one VorbisReader per stream.
 using System;
 using System.Buffers;
@@ -97,6 +97,72 @@ namespace NVorbis.Gpu
                 if (rc < 0) dst.Dispose();
                 Vpz.Check(rc, gpu.Handle);
                 return (dst, offsets, got);
+            }
+        }
+
+        /// <summary>Elements (fp32, or int16 with int16: true) a DecodeFilesToDevice call of these files writes, and the
+        /// samples per channel of each file: the size query, nothing is decoded.</summary>
+        public static long DeviceElements(GpuContext gpu, ReadOnlyMemory<byte>[] files, out long[] sampleCounts, bool clip = true)
+        {
+            using PinnedImages im = new(files);
+            sampleCounts = new long[files.Length];
+            fixed (IntPtr* p = im.Ptrs)
+            fixed (nuint* l = im.Lens)
+            fixed (long* c = sampleCounts)
+            {
+                long total = Vpz.vpz_decode_files_device(gpu.Handle, (uint)files.Length, (byte**)p, l, clip ? 1 : 0, 0, IntPtr.Zero, 0, c, IntPtr.Zero);
+                Vpz.Check(total, gpu.Handle);
+                return total;
+            }
+        }
+
+        /// <summary>DecodeFiles with the PCM left in GPU memory: dstDevice is device memory of the context's GPU with room
+        /// for dstElements elements (DeviceElements); file k starts at element sum over j &lt; k of samples_j * channels_j,
+        /// channel-major [channels][samples] with planar: true, interleaved otherwise; int16: the rule of DecodeFilesInt16,
+        /// for every stream.  The call waits for the work queued on `stream` (a cudaStream_t, IntPtr.Zero: the legacy
+        /// default stream) and returns when dstDevice is complete.  Returns the samples per channel of each file.</summary>
+        public static long[] DecodeFilesToDevice(GpuContext gpu, ReadOnlyMemory<byte>[] files, IntPtr dstDevice, long dstElements,
+                                                 bool planar = true, bool int16 = false, bool clip = true, IntPtr stream = default)
+        {
+            using PinnedImages im = new(files);
+            long[] counts = new long[files.Length];
+            int format = (planar ? Vpz.OutPlanar : 0) | (int16 ? Vpz.OutS16 : 0);
+            fixed (IntPtr* p = im.Ptrs)
+            fixed (nuint* l = im.Lens)
+            fixed (long* c = counts)
+            {
+                Vpz.Check(Vpz.vpz_decode_files_device(gpu.Handle, (uint)files.Length, (byte**)p, l, clip ? 1 : 0, format, dstDevice,
+                                                      (nuint)dstElements, c, stream), gpu.Handle);
+                return counts;
+            }
+        }
+
+        /// <summary>ReadExcerpts with the PCM left in GPU memory (layout, format and stream as DecodeFilesToDevice; excerpt i
+        /// holds count samples per channel at element offsets[i], undelivered samples are 0).  dstDevice == IntPtr.Zero:
+        /// only the layout is computed.  Returns the total elements of the layout.</summary>
+        public static long ReadExcerptsToDevice(GpuContext gpu, ReadOnlyMemory<byte>[] files, (int file, long start, int count)[] excerpts,
+                                                IntPtr dstDevice, long dstElements, out long[] offsets, out int[] got,
+                                                bool planar = true, bool int16 = false, bool clip = true, IntPtr stream = default)
+        {
+            using PinnedImages im = new(files);
+            int n = excerpts.Length;
+            uint[] fileOf = new uint[Math.Max(n, 1)];
+            long[] start = new long[Math.Max(n, 1)];
+            int[] count = new int[Math.Max(n, 1)];
+            for (int i = 0; i < n; i++) (fileOf[i], start[i], count[i]) = ((uint)excerpts[i].file, excerpts[i].start, excerpts[i].count);
+            offsets = new long[Math.Max(n, 1)];
+            got = new int[Math.Max(n, 1)];
+            int format = (planar ? Vpz.OutPlanar : 0) | (int16 ? Vpz.OutS16 : 0);
+            fixed (IntPtr* p = im.Ptrs)
+            fixed (nuint* l = im.Lens)
+            fixed (uint* f = fileOf)
+            fixed (long* s = start, o = offsets)
+            fixed (int* c = count, g = got)
+            {
+                long rc = Vpz.vpz_decode_excerpts_device(gpu.Handle, (uint)files.Length, (byte**)p, l, (uint)n, f, s, c, clip ? 1 : 0, format,
+                                                         dstDevice, (nuint)dstElements, o, g, stream);
+                Vpz.Check(rc, gpu.Handle);
+                return rc;
             }
         }
 

@@ -134,6 +134,10 @@ namespace NVorbis.Gpu
         [LibraryImport(Lib)] internal static partial long vpz_decode_files_s16(IntPtr ctx, uint n, byte** datas, nuint* lens, int clip, short* dst, nuint dstSamples, long* sampleCounts);
         [LibraryImport(Lib)] internal static partial long vpz_scan_pages(IntPtr ctx, uint n, byte** datas, nuint* lens, VpzPageInfo* pages, nuint pagesCap, uint* first, uint* count, ulong* wasteBits, uint* crcFailures);
         [LibraryImport(Lib)] internal static partial long vpz_decode_excerpts(IntPtr ctx, uint nFiles, byte** datas, nuint* lens, uint n, uint* fileOf, long* start, int* count, int clip, float* dst, nuint dstFloats, long* dstOffsets, int* got);
+        // format bits of the *_device calls (0 = fp32 interleaved); dstDev is device memory of the context's GPU, stream a cudaStream_t
+        internal const int OutS16 = 1, OutPlanar = 2;
+        [LibraryImport(Lib)] internal static partial long vpz_decode_files_device(IntPtr ctx, uint n, byte** datas, nuint* lens, int clip, int format, IntPtr dstDev, nuint dstElems, long* sampleCounts, IntPtr stream);
+        [LibraryImport(Lib)] internal static partial long vpz_decode_excerpts_device(IntPtr ctx, uint nFiles, byte** datas, nuint* lens, uint n, uint* fileOf, long* start, int* count, int clip, int format, IntPtr dstDev, nuint dstElems, long* dstOffsets, int* got, IntPtr stream);
         [LibraryImport(Lib)] internal static partial long vpz_debug_page_end_granules(IntPtr ctx, byte* data, nuint len, int onDevice, long* dst, nuint cap);
     }
 }

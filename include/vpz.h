@@ -70,7 +70,8 @@ int vpz_device_count(void);
  * at this many MiB of container images, default 128, at most 384),
  * "host_threads" (size of the host worker pool of the bulk calls, default 0 = all cores up to 32), "bulk_threads"
  * (how many of them vpz_decode_files uses, default 4: the call is bound by the PCM copy, which more staging
- * threads slow down; 0 = all), "gpu_scan" (bulk
+ * threads slow down; 0 = all), "bulk_threads_device" (the same for vpz_decode_files_device, default 8: without a
+ * PCIe copy the call is bound by the host's scan and planning, and 8 threads measured fastest), "gpu_scan" (bulk
  * path: Ogg page scan + CRC on the GPU, default 1), "force_general" (tests: route every packet through the
  * general kernels). */
 int vpz_ctx_set(vpz_ctx* ctx, const char* key, int value);
@@ -313,6 +314,33 @@ int64_t vpz_scan_pages(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, co
 int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
                             uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
                             int clip, float* dst, size_t dst_floats, int64_t* dst_offsets, int32_t* got);
+
+/* ---- bulk calls with the PCM in caller-owned device memory ----------------------------------------- */
+/* Format bits of the *_device calls; 0 = fp32 interleaved (the host calls' layout). */
+enum { VPZ_OUT_S16 = 1, VPZ_OUT_PLANAR = 2 };
+
+/* vpz_decode_files / vpz_decode_excerpts with the samples written to dst_dev, device (or managed) memory of
+ * the context's device, instead of host memory.  What is decoded, sample_counts / got / dst_offsets, the size
+ * query (dst_dev == NULL), the errors and ClipSamples are those of the host calls.  Item k (file k, excerpt k)
+ * starts at ELEMENT offset dst_offsets[k], the host calls' offsets; dst_elems and the offsets count elements
+ * (4 bytes for fp32, 2 for VPZ_OUT_S16).
+ *   VPZ_OUT_PLANAR: item k is channel-major, channel c at dst_offsets[k] + c * samples_k (samples_k = sample_counts[k]
+ *                   for files, count[k] for excerpts); items of one channel count and one length make a dense
+ *                   [n][C][T] array.  Without it, items are interleaved.
+ *   VPZ_OUT_S16:    int16 elements, v = (int)(x * 32768f) clamped to [-32768, 32767] after ClipSamples, for every
+ *                   stream the fp32 path decodes (any channel count and block size).
+ * Samples an excerpt does not deliver (end of stream, failed SeekTo) are zero.  stream: the caller's cudaStream_t
+ * (NULL: the legacy default stream); the library's work starts after the work queued on it before the call, and
+ * dst_dev is complete when the call returns.  A host, pinned or other-device pointer, a too small dst_elems and
+ * unknown format bits fail with VPZ_E_ARGUMENT.  The PCM is placed by one more kernel pass over the batch PCM
+ * (K5) instead of a device-to-host copy; "bulk_threads_device" sets the host threads of the files call. */
+int64_t vpz_decode_files_device(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens,
+                                int clip, int format, void* dst_dev, size_t dst_elems,
+                                int64_t* sample_counts, void* stream);
+int64_t vpz_decode_excerpts_device(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
+                                   uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
+                                   int clip, int format, void* dst_dev, size_t dst_elems,
+                                   int64_t* dst_offsets, int32_t* got, void* stream);
 
 /* Debug / tests: the page-end granule index SeekTo searches in (PacketProvider.FillPageEndGranuleCache,
  * Ogg/PacketProvider.cs:203-307) of one container image's first logical stream: entry p = granules up to and

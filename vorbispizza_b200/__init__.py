@@ -16,9 +16,12 @@ from .api import (  # noqa: F401
     SynthBatch,
     VorbisReader,
     decode_excerpts,
+    decode_excerpts_device,
     decode_files,
+    decode_files_device,
     scan_pages,
 )
 
-__all__ = ["Batch", "Context", "SynthBatch", "VorbisReader", "decode_files", "decode_excerpts", "scan_pages", "VpzError", "InvalidDataError",
+__all__ = ["Batch", "Context", "SynthBatch", "VorbisReader", "decode_files", "decode_excerpts", "decode_files_device",
+           "decode_excerpts_device", "scan_pages", "VpzError", "InvalidDataError",
            "SeekOutOfRangeError", "PreRollPacketError", "load"]

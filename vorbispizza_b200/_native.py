@@ -26,6 +26,9 @@ VPZ_E_REF_FAULT = -11
 
 DUMP_MAX_CH = 8
 
+VPZ_OUT_S16 = 1      # format bits of the *_device bulk calls; 0 = fp32 interleaved
+VPZ_OUT_PLANAR = 2
+
 
 class SetupInfo(C.Structure):
     _fields_ = [("channels", C.c_int32), ("sample_rate", C.c_int32), ("bitrate_upper", C.c_int32),
@@ -120,7 +123,10 @@ _SIGS = {
     "vpz_decode_files": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_int, _P, C.c_size_t, _P]),
     "vpz_decode_files_s16": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_int, _P, C.c_size_t, _P]),
     "vpz_decode_excerpts": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_uint32, _P, _P, _P, C.c_int, _P, C.c_size_t, _P, _P]),
-    "vpz_debug_page_end_granules": (C.c_int64, [_P, _P, C.c_size_t, C.c_int, _P, C.c_size_t]),
+    "vpz_decode_files_device": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_int, C.c_int, _P, C.c_size_t, _P, _P]),
+    "vpz_decode_excerpts_device": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_uint32, _P, _P, _P, C.c_int, C.c_int, _P,
+                                               C.c_size_t, _P, _P, _P]),
+    "vpz_debug_page_end_granules":(C.c_int64, [_P, _P, C.c_size_t, C.c_int, _P, C.c_size_t]),
     "vpz_scan_pages": (C.c_int64, [_P, C.c_uint32, _P, _P, _P, C.c_size_t, _P, _P, _P, _P]),
 }
 

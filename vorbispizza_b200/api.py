@@ -45,6 +45,7 @@ class Context:
 
     def __init__(self, device=-1, lib_path=None):
         self.lib = N.load(lib_path)
+        self.device = device
         h = C.c_void_p()
         rc = self.lib.vpz_ctx_create(device, C.byref(h))
         if rc:
@@ -487,6 +488,95 @@ def decode_excerpts(ctx, files, file_of, start, count, clip=True, dst=None):
         dst = np.full(total, np.nan, np.float32)   # the call defines every float: short reads are zero-filled
     total = ctx.check(ctx.lib.vpz_decode_excerpts(*args, dst.ctypes.data, dst.size, offsets.ctypes.data, got.ctypes.data))
     return dst[:total], offsets, got
+
+
+def _device_out(ctx, out, total, dtype, stream):
+    """The destination of a *_device call: (buffer, pointer, elements, cudaStream_t handle).  out=None allocates a
+    torch CUDA tensor on the context's device; out may be a caller tensor, or a numpy array for the emulated
+    library (whose device memory is host memory).  stream=None: torch's current stream for a tensor."""
+    if dtype not in ("float32", "int16"):
+        raise ValueError("dtype must be 'float32' or 'int16'")
+    if out is None:
+        import torch
+        dev = torch.device("cuda", ctx.device if ctx.device >= 0 else torch.cuda.current_device())
+        out = torch.empty(max(total, 1), dtype=getattr(torch, dtype), device=dev)[:total]
+    if isinstance(out, np.ndarray):
+        if out.dtype != np.dtype(dtype) or not out.flags.c_contiguous:
+            raise ValueError("out must be a contiguous %s array" % dtype)
+        return out, (out.ctypes.data if out.size else None), out.size, stream
+    import torch
+    if out.dtype != getattr(torch, dtype) or not out.is_contiguous():
+        raise ValueError("out must be a contiguous %s tensor" % dtype)
+    if stream is None and out.is_cuda:
+        stream = torch.cuda.current_stream(out.device)
+    handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else stream
+    return out, (out.data_ptr() if out.numel() else None), out.numel(), handle
+
+
+def _format(dtype, planar):
+    return (N.VPZ_OUT_S16 if dtype == "int16" else 0) | (N.VPZ_OUT_PLANAR if planar else 0)
+
+
+def _vorbis_channels(data):
+    """Channel count from a container image's first identification header ("\\x01vorbis", channels at byte 11)."""
+    i = bytes(data[:1 << 16]).find(b"\x01vorbis")
+    return data[i + 11] if i >= 0 and i + 11 < len(data) else 0
+
+
+def decode_files_device(ctx, files, clip=True, dtype="float32", planar=True, out=None, stream=None):
+    """vpz_decode_files_device: decode_files with the PCM left in device memory.
+
+    Returns (buf, offsets, counts): buf is one flat buffer of `dtype` ("float32", or "int16" by the reference
+    tests' (int)(x * 32768f) rule); file k starts at element offsets[k] and has counts[k] samples per channel,
+    channel-major [C_k][counts[k]] with planar=True, interleaved otherwise.  When every file has the same channel
+    count C and length T, ``buf.view(n, C, T)`` is the batch.  out: a caller tensor (contiguous, on the context's
+    device) instead of a new one; stream: the torch / CUDA stream the result is used on (default: the current one);
+    the call waits for the work queued on it and returns when buf is complete."""
+    keep = [_u8(f) for f in files]
+    n = len(keep)
+    ptrs = (C.c_void_p * n)(*[k[1] for k in keep])
+    lens = (C.c_size_t * n)(*[k[2] for k in keep])
+    counts = np.zeros(n, np.int64)
+    fmt = _format(dtype, planar)
+    args = (ctx._h, n, ptrs, lens, int(bool(clip)), fmt)
+    total = None
+    if out is None:
+        total = ctx.check(ctx.lib.vpz_decode_files_device(*args, None, 0, counts.ctypes.data, None))
+    buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
+    total = ctx.check(ctx.lib.vpz_decode_files_device(*args, ptr, elems, counts.ctypes.data, handle))
+    chans = np.array([_vorbis_channels(k[0]) for k in keep], np.int64)
+    offsets = np.zeros(n, np.int64)
+    if n > 1:
+        offsets[1:] = np.cumsum(counts * chans)[:-1]
+    return buf[:total], offsets, counts
+
+
+def decode_excerpts_device(ctx, files, file_of, start, count, clip=True, dtype="float32", planar=True, out=None,
+                           stream=None):
+    """vpz_decode_excerpts_device: decode_excerpts with the PCM left in device memory.
+
+    Returns (buf, offsets, got) as decode_excerpts does; excerpt i starts at element offsets[i] and holds count[i]
+    samples per channel, channel-major with planar=True; samples not delivered are zero.  With one channel count C
+    and a uniform count T (a crop batch), ``buf.view(n, C, T)`` is the batch.  dtype, out, stream: as
+    decode_files_device."""
+    keep = [_u8(f) for f in files]
+    nf = len(keep)
+    ptrs = (C.c_void_p * nf)(*[k[1] for k in keep])
+    lens = (C.c_size_t * nf)(*[k[2] for k in keep])
+    file_of = np.ascontiguousarray(file_of, dtype=np.uint32)
+    start = np.ascontiguousarray(start, dtype=np.int64)
+    count = np.ascontiguousarray(count, dtype=np.int32)
+    n = file_of.size
+    offsets = np.zeros(n, np.int64)
+    got = np.zeros(n, np.int32)
+    args = (ctx._h, nf, ptrs, lens, n, file_of.ctypes.data, start.ctypes.data, count.ctypes.data, int(bool(clip)),
+            _format(dtype, planar))
+    total = None
+    if out is None:
+        total = ctx.check(ctx.lib.vpz_decode_excerpts_device(*args, None, 0, offsets.ctypes.data, got.ctypes.data, None))
+    buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
+    total = ctx.check(ctx.lib.vpz_decode_excerpts_device(*args, ptr, elems, offsets.ctypes.data, got.ctypes.data, handle))
+    return buf[:total], offsets, got
 
 
 PAGE_DTYPE = np.dtype([("offset", "<u4"), ("body_len", "<u4"), ("granule", "<i8"), ("serial", "<u4"), ("sequence", "<u4"),

@@ -11,6 +11,7 @@
 #include "k1_symbols.cuh"
 #include "k3_streams.cuh"
 #include "k4_deliver.cuh"
+#include "k5_place.cuh"
 
 // ---- kernels ---------------------------------------------------------------------------------
 __global__ void __launch_bounds__(K0_THREADS) vpz_k0_pages(K0Params P) {
@@ -26,6 +27,9 @@ __global__ void __launch_bounds__(K0_THREADS) vpz_k0_crc(K0Params P) {
 __global__ void __launch_bounds__(K0_THREADS) vpz_k0g_granules(K0gParams P) { k0g_cta(P); }
 
 __global__ void __launch_bounds__(K4_THREADS) vpz_k4_deliver(K4Params P) { k4_cta(P); }
+
+template <bool OUT16, bool PLANAR>
+__global__ void __launch_bounds__(K5_THREADS) vpz_k5_place(K5Params P) { k5_cta<OUT16, PLANAR>(P); }
 
 #ifndef K1A_MIN_CTAS
 #define K1A_MIN_CTAS 8
@@ -303,6 +307,41 @@ int launch_k4(const K4Params& p, Stream* s, std::string& err) {
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k4_deliver", err);
 }
+
+int launch_k5(const K5Params& p, Stream* s, std::string& err) {
+  if (p.n_tiles == 0) return VPZ_OK;
+  const unsigned warps = K5_THREADS / 32;
+  unsigned grid = (unsigned)std::min<size_t>(((size_t)p.n_tiles + warps - 1) / warps, (size_t)8 * sm_count());
+  if (p.out16) {
+    if (p.planar) vpz_k5_place<true, true><<<grid, K5_THREADS, 0, s->s>>>(p); else vpz_k5_place<true, false><<<grid, K5_THREADS, 0, s->s>>>(p);
+  } else {
+    if (p.planar) vpz_k5_place<false, true><<<grid, K5_THREADS, 0, s->s>>>(p); else vpz_k5_place<false, false><<<grid, K5_THREADS, 0, s->s>>>(p);
+  }
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k5_place", err);
+}
+
+int check_device_ptr(const void* p, int device, std::string& err) {
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, p);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    err = std::string("destination: cudaPointerGetAttributes: ") + cudaGetErrorString(e);
+    return VPZ_E_ARGUMENT;
+  }
+  if (a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) {
+    err = a.type == cudaMemoryTypeHost ? "destination is pinned host memory, not device memory"
+                                       : "destination is not CUDA device memory";
+    return VPZ_E_ARGUMENT;
+  }
+  if (a.type == cudaMemoryTypeDevice && a.device != device) {
+    err = "destination is memory of device " + std::to_string(a.device) + ", the context's device is " + std::to_string(device);
+    return VPZ_E_ARGUMENT;
+  }
+  return VPZ_OK;
+}
+
+void event_record_external(Event* e, void* cuda_stream) { cudaEventRecord(e->e, static_cast<cudaStream_t>(cuda_stream)); }
 
 int launch_k1a(const K1Params& p, bool debug, bool full, int blocks, Stream* s, std::string& err) {
   if (p.n_pkts == 0) return VPZ_OK;

@@ -68,6 +68,14 @@ int launch_k0(const K0Params& p, Stream* s, std::string& err);
 int launch_k0g(const K0gParams& p, Stream* s, std::string& err);
 // K4: copy segments of decoded excerpts into the caller's layout, one warp per segment
 int launch_k4(const K4Params& p, Stream* s, std::string& err);
+// K5: tiles of the batch PCM into the caller's device buffer, one warp per tile
+int launch_k5(const K5Params& p, Stream* s, std::string& err);
+
+// Caller-owned device memory (the *_device bulk calls): 0 when p is device or managed memory of `device`,
+// VPZ_E_ARGUMENT (with the reason in err) for host, pinned or another device's memory
+int check_device_ptr(const void* p, int device, std::string& err);
+// Records e on the caller's cudaStream_t (NULL: the legacy default stream)
+void event_record_external(Event* e, void* cuda_stream);
 size_t max_smem_per_block();             // of the calling thread's current device
 
 }  // namespace dev

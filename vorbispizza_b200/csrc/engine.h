@@ -67,6 +67,7 @@ class ThreadPool {
 
 namespace vpz {
 struct ExcerptBufs;                  // below: buffers of the bulk random-access path (K4)
+struct PlaceBufs;                    // below: tiles of the device-output bulk calls (K5)
 struct ScanBufs;                     // scan.cpp: staging of the device page scan (K0)
 void scan_bufs_destroy(ScanBufs* s);
 struct ScanResult {                  // views into the context's scan buffers, valid until the next scan
@@ -103,11 +104,13 @@ struct vpz_ctx {
   vpz::dev::Event* bulk_done[3] = {nullptr, nullptr, nullptr};   // D2H of the batch's PCM finished
   vpz::dev::Event* bulk_ready[3] = {nullptr, nullptr, nullptr};  // kernels of the batch finished
   vpz::ExcerptBufs* xb = nullptr;            // vpz_decode_excerpts: copy segments and dense output of the two groups in flight
+  vpz::PlaceBufs* place = nullptr;           // *_device bulk calls: K5 tiles of the groups in flight
   int bulk_group = 256;                      // streams per pipeline group ("bulk_group" tunable)
   int bulk_group_mib = 128;                  // ... and at most this many MiB of container images ("bulk_group_mib")
   int bulk_group_bytes = 0;                  // tests: the same limit in bytes (overrides bulk_group_mib when > 0)
   int host_threads = 0;                      // size of the worker pool; 0: hardware concurrency, capped at 32
   int bulk_threads = 4;                      // of those, how many vpz_decode_files uses ("bulk_threads"; 0: all)
+  int bulk_threads_device = 8;               // ... and vpz_decode_files_device ("bulk_threads_device"; 0: all)
 };
 
 namespace vpz {
@@ -165,6 +168,11 @@ struct ExcerptBufs {
       dev::event_destroy(done[i]);
     }
   }
+};
+
+struct PlaceBufs {   // one slot per pipeline batch (vpz_decode_files_device: 3, vpz_decode_excerpts_device: 2)
+  HostBuf<VpzPlaceTile> h_tiles[3];
+  DevBuf d_tiles[3];
 };
 
 struct PktSrc {

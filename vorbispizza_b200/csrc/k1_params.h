@@ -69,6 +69,16 @@ struct K4Params {
   int clip;
 };
 
+struct K5Params {
+  const float* pcm;                // batch PCM (K3 output)
+  void* out;                       // the caller's device buffer: fp32 or int16 elements
+  const VpzPlaceTile* tiles;
+  uint32_t n_tiles;
+  int planar;                      // 1: channel-major items, 0: interleaved
+  int out16;                       // 1: int16 elements by K3's rule (k3_s16)
+  int clip;                        // clip before the conversion (the excerpt path decodes unclipped)
+};
+
 struct K0gParams {
   const uint8_t* images;           // the staged images of the K0 scan
   const VpzGranFile* files;

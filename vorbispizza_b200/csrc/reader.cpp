@@ -871,9 +871,102 @@ struct BulkJob {
 
 }  // extern "C"
 
+// ---- device output (vpz_decode_files_device, vpz_decode_excerpts_device) --------------------------
+// The bulk pipelines stay as they are; only the last step of a group differs: instead of a device->host copy of
+// the group's PCM, K5 places tiles of the batch PCM into the caller's device buffer on the compute stream.
+namespace {
+struct DevOut {
+  void* p = nullptr;       // the caller's device buffer (NULL: size query)
+  int format = 0;          // VPZ_OUT_* bits
+  void* stream = nullptr;  // the caller's cudaStream_t
+};
+
+size_t tile_count(uint64_t samples) { return (size_t)((samples + VPZ_TILE_SAMPLES - 1) / VPZ_TILE_SAMPLES); }
+
+// samples [first, first + n) of an item (element base `base`, `len` samples per channel, `ch` channels) from the
+// batch PCM at float offset src (VPZ_TILE_ZERO: zeros), cut into tiles; returns the end of the written tiles
+VpzPlaceTile* put_tiles(VpzPlaceTile* out, uint64_t src, uint64_t base, uint64_t len, uint64_t first, uint64_t n, uint32_t ch) {
+  for (uint64_t s = 0; s < n; s += VPZ_TILE_SAMPLES) {
+    VpzPlaceTile t;
+    t.src = src == VPZ_TILE_ZERO ? src : src + s * ch;
+    t.base = base;
+    t.len = len;
+    t.first = first + s;
+    t.n = (uint32_t)std::min<uint64_t>(VPZ_TILE_SAMPLES, n - s);
+    t.ch = ch;
+    *out++ = t;
+  }
+  return out;
+}
+void append_tiles(std::vector<VpzPlaceTile>& v, uint64_t src, uint64_t base, uint64_t len, uint64_t first, uint64_t n, uint32_t ch) {
+  const size_t at = v.size();
+  v.resize(at + tile_count(n));
+  put_tiles(v.data() + at, src, base, len, first, n, ch);
+}
+
+// Checks the destination and orders the context's stream behind the work already queued on the caller's stream
+// (a tensor from a caching allocator may still be in use there); *ev is destroyed by device_output_end
+int device_output_begin(vpz_ctx* ctx, const DevOut& o, dev::Event** ev) {
+  if (o.format & ~(VPZ_OUT_S16 | VPZ_OUT_PLANAR)) {
+    ctx->last_error = "unknown output format bits";
+    return VPZ_E_ARGUMENT;
+  }
+  if (!o.p) return VPZ_OK;   // size query
+  int rc = dev::check_device_ptr(o.p, ctx->device, ctx->last_error);
+  if (rc) return rc;
+  if (!ctx->place) {
+    ctx->place = new (std::nothrow) PlaceBufs;
+    if (!ctx->place) return VPZ_E_NOMEM;
+  }
+  *ev = dev::event_create();
+  if (!*ev) {
+    ctx->last_error = "cudaEventCreate failed";
+    return VPZ_E_CUDA;
+  }
+  dev::event_record_external(*ev, o.stream);
+  dev::stream_wait_event(ctx->stream, *ev);
+  return VPZ_OK;
+}
+// Nothing of the call stays queued behind it: the destination is complete when the call returns
+int64_t device_output_end(vpz_ctx* ctx, dev::Event* ev, int64_t rc) {
+  if (!ev) return rc;
+  std::string err;
+  int r2 = dev::stream_sync(ctx->stream, err);
+  dev::event_destroy(ev);
+  if (r2 && rc >= 0) {
+    ctx->last_error = err;
+    return r2;
+  }
+  return rc;
+}
+
+// Uploads the tiles of pipeline slot `slot` and launches K5 on the context's stream
+int place_tiles(vpz_ctx* ctx, int slot, const vpz_batch* b, const DevOut& o, int clip) {
+  PlaceBufs& pb = *ctx->place;
+  const size_t n = pb.h_tiles[slot].n;
+  if (!n) return VPZ_OK;
+  if (!pb.d_tiles[slot].reserve(n * sizeof(VpzPlaceTile), ctx->last_error)) return VPZ_E_CUDA;
+  int rc = dev::h2d(pb.d_tiles[slot].p, pb.h_tiles[slot].p, n * sizeof(VpzPlaceTile), ctx->stream, ctx->last_error);
+  if (rc) return rc;
+  K5Params kp;
+  kp.pcm = static_cast<const float*>(b->d_pcm.p);
+  kp.out = o.p;
+  kp.tiles = static_cast<const VpzPlaceTile*>(pb.d_tiles[slot].p);
+  kp.n_tiles = (uint32_t)n;
+  kp.planar = (o.format & VPZ_OUT_PLANAR) ? 1 : 0;
+  kp.out16 = (o.format & VPZ_OUT_S16) ? 1 : 0;
+  kp.clip = clip ? 1 : 0;
+  rc = dev::launch_k5(kp, ctx->stream, ctx->last_error);
+  if (!rc) ctx->kernel_launches++;
+  return rc;
+}
+}  // namespace
+
 // out16: dst holds int16 elements (same element offsets), produced on the GPU by K3
+// dout: the caller's device buffer instead (dst is its address): K3 writes fp32, K5 places and converts
 static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int clip,
-                                 float* dst, size_t dst_floats, int64_t* sample_counts, int out16) {
+                                 float* dst, size_t dst_floats, int64_t* sample_counts, int out16,
+                                 const DevOut* dout = nullptr) {
   if (!ctx || (n && (!datas || !lens))) return VPZ_E_ARGUMENT;
   VPZ_USE(ctx);
   if (!ctx->pool) {
@@ -885,12 +978,13 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
   ThreadPool* pool = ctx->pool;
   // The call is bound by the PCM copy, and the copy gets SLOWER the more host threads stage packets beside it
   // (16-core box, 4,096 streams: 2 / 4 / 8 / 16 threads = 169 / 167 / 171 / 178 ms; with 2 the 16-bit path turns
-  // host-bound): a few threads are the optimum, "bulk_threads" (default 4).
+  // host-bound): a few threads are the optimum, "bulk_threads" (default 4).  The device-output call has no PCIe
+  // copy to slow down: "bulk_threads_device".
   struct PoolLimit {
     ThreadPool* p;
     PoolLimit(ThreadPool* pool_, unsigned k) : p(pool_) { p->set_limit(k); }
     ~PoolLimit() { p->set_limit(0); }
-  } pool_limit(pool, (unsigned)std::max(0, ctx->bulk_threads));
+  } pool_limit(pool, (unsigned)std::max(0, dout ? ctx->bulk_threads_device : ctx->bulk_threads));
   const bool trace = getenv("VPZ_TRACE") != nullptr;
   double t_scan = 0, t_init = 0, t_plan = 0, t_commit = 0, t_launch = 0, t_wait = 0;
   auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
@@ -1020,8 +1114,35 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
       rc = VPZ_E_INVALID_OP;
       break;
     }
+    if (dout && group_floats) {
+      // 4b. K5 tiles: file i of the group is the batch PCM at its offset in the group (runs are committed in
+      //     file order), placed at element total + that offset
+      std::vector<uint64_t> off(cnt + 1, 0);
+      std::vector<size_t> first_tile(cnt + 1, 0);
+      for (uint32_t i = 0; i < cnt; i++) {
+        const BulkJob& j = *jobs[i];
+        const int64_t samples = j.win.has_plan ? j.win.plan.samples : 0;
+        off[i + 1] = off[i] + (uint64_t)samples * j.dec.channels();
+        first_tile[i + 1] = first_tile[i] + tile_count((uint64_t)samples);
+      }
+      HostBuf<VpzPlaceTile>& ht = ctx->place->h_tiles[slot];
+      if (!ht.reserve(first_tile[cnt])) {
+        rc = VPZ_E_NOMEM;
+        break;
+      }
+      ht.n = first_tile[cnt];
+      pool->parallel_for(cnt, [&](size_t i) {
+        const BulkJob& j = *jobs[i];
+        const uint64_t samples = j.win.has_plan ? (uint64_t)j.win.plan.samples : 0;
+        put_tiles(ht.p + first_tile[i], off[i], (uint64_t)total + off[i], samples, 0, samples, (uint32_t)j.dec.channels());
+      });
+    }
     t1 = now(); t_commit += t1 - t0; t0 = t1;
-    if (group_floats) {
+    if (group_floats && dout) {
+      // 5. H2D + K1 + K3 + K5 (batch PCM -> the caller's device buffer) on the compute stream
+      if ((rc = batch_decode(b, clip, 0))) break;
+      if ((rc = place_tiles(ctx, slot, b, *dout, 0))) break;   // (K3 has clipped)
+    } else if (group_floats) {
       // 5. H2D + K1 + K3 on the compute stream, then the PCM of this group on the copy stream
       if ((rc = batch_decode(b, clip, out16))) break;
       dev::event_record(ctx->bulk_ready[slot], ctx->stream);
@@ -1032,7 +1153,7 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
         rc = dev::d2h(dst + total, b->d_pcm.p, group_floats * 4, ctx->copy_stream, ctx->last_error);
       if (rc) break;
     }
-    dev::event_record(ctx->bulk_done[slot], ctx->copy_stream);
+    dev::event_record(ctx->bulk_done[slot], dout ? ctx->stream : ctx->copy_stream);
     t1 = now(); t_launch += t1 - t0; t0 = t1;
     used[slot] = true;
     total += (int64_t)group_floats;
@@ -1050,8 +1171,8 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
       if (ctx->bulk[s]) vpz_batch_reset(ctx->bulk[s]);  // drop setup references; device buffers stay allocated
   }
   if (trace) {
-    fprintf(stderr, "vpz_decode_files: %u files, %u groups: scan %.1f init %.1f plan %.1f commit %.1f launch %.1f wait %.1f drain %.1f ms\n",
-            n, group, t_scan, t_init, t_plan, t_commit, t_launch, t_wait, now() - t0);
+    fprintf(stderr, "vpz_decode_files%s: %u files, %u groups: scan %.1f init %.1f plan %.1f commit %.1f launch %.1f wait %.1f drain %.1f ms\n",
+            dout ? "_device" : "", n, group, t_scan, t_init, t_plan, t_commit, t_launch, t_wait, now() - t0);
     fprintf(stderr, "  inside launch (cumulative): order sort %.1f, upload incl. sort %.1f, kernel launches %.1f ms\n",
             vpz::g_trace_ms[0], vpz::g_trace_ms[1], vpz::g_trace_ms[2]);
   }
@@ -1068,6 +1189,21 @@ int64_t vpz_decode_files(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, 
 int64_t vpz_decode_files_s16(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int clip,
                              int16_t* dst, size_t dst_samples, int64_t* sample_counts) {
   return decode_files_impl(ctx, n, datas, lens, clip, reinterpret_cast<float*>(dst), dst_samples, sample_counts, 1);
+}
+
+int64_t vpz_decode_files_device(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int clip,
+                                int format, void* dst_dev, size_t dst_elems, int64_t* sample_counts, void* stream) {
+  if (!ctx || (n && (!datas || !lens))) return VPZ_E_ARGUMENT;
+  VPZ_USE(ctx);
+  DevOut o;
+  o.p = dst_dev;
+  o.format = format;
+  o.stream = stream;
+  dev::Event* ev = nullptr;
+  int rc = device_output_begin(ctx, o, &ev);
+  if (rc) return device_output_end(ctx, ev, rc);
+  return device_output_end(ctx, ev, decode_files_impl(ctx, n, datas, lens, clip, static_cast<float*>(dst_dev), dst_elems,
+                                                      sample_counts, 0, &o));
 }
 
 
@@ -1205,11 +1341,13 @@ static int open_excerpt_files(vpz_ctx* ctx, uint32_t n_files, const uint8_t* con
   return VPZ_OK;
 }
 
-int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens, uint32_t n,
-                            const uint32_t* file_of, const int64_t* start, const int32_t* count, int clip, float* dst,
-                            size_t dst_floats, int64_t* dst_offsets, int32_t* got) {
-  if (!ctx || !datas || !lens || (n && (!file_of || !start || !count))) return VPZ_E_ARGUMENT;
-  VPZ_USE(ctx);
+}  // extern "C"
+
+// dout: the caller's device buffer instead of dst (dst is its address): K5 places the segments and zero-fills
+static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
+                                    uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
+                                    int clip, float* dst, size_t dst_floats, int64_t* dst_offsets, int32_t* got,
+                                    const DevOut* dout) {
   if (!ctx->pool) {
     unsigned t = ctx->host_threads > 0 ? (unsigned)ctx->host_threads
                                        : std::max(1u, std::min(std::thread::hardware_concurrency(), 32u));
@@ -1354,6 +1492,7 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
   int rc = VPZ_OK;
   bool used[2] = {false, false};
   std::vector<std::vector<VpzCopySeg>> task_segs;
+  std::vector<std::vector<VpzPlaceTile>> task_tiles;
   for (size_t gi = 0; gi < groups.size() && !rc; gi++) {
     const Group& g = groups[gi];
     const int slot = (int)(gi & 1);
@@ -1396,6 +1535,7 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
     tt1 = now(); t_commit += tt1 - tt0; tt0 = tt1;
     // consumer side, samples untouched: SeekTo's two packets, then Read until `count` samples or the end
     task_segs.assign(g.t1 - g.t0, std::vector<VpzCopySeg>());
+    if (dout) task_tiles.assign(g.t1 - g.t0, std::vector<VpzPlaceTile>());
     pool->parallel_for(g.t1 - g.t0, [&](size_t k) {
       ExcerptTask& t = tasks[g.t0 + k];
       StreamDec* d = t.dec.get();
@@ -1406,11 +1546,13 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
         const uint32_t i = j.index;
         if (j.status) {
           if (got) got[i] = j.status;
+          if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
           continue;
         }
         int prc = place_window(d, b, j.win.get(), j.run, j.drain_run, 0);
         if (prc) {
           if (got) got[i] = prc;
+          if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
           continue;
         }
         d->current_position = 0;
@@ -1438,6 +1580,12 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
         }
         d->seg_sink = nullptr;
         if (got) got[i] = src ? src : have;
+        if (dout) {   // the segments (samples [0, have)), then zeros up to count
+          const uint64_t item = (uint64_t)(dst_offsets[i] - g.base);
+          for (size_t sg = mark; sg < segs.size(); sg++)
+            append_tiles(task_tiles[k], segs[sg].src, dst_offsets[i], count[i], (segs[sg].dst - item) / C, segs[sg].n / C, C);
+          append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], have, count[i] - have, C);
+        }
         j.win.reset();   // release the packet views / arena
       }
     });
@@ -1455,7 +1603,33 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
       }
       xb.h_segs[slot].n = n_segs;
     }
+    if (dout) {
+      size_t n_tiles = 0;
+      for (const auto& v : task_tiles) n_tiles += v.size();
+      HostBuf<VpzPlaceTile>& ht = ctx->place->h_tiles[slot];
+      if (!ht.reserve(n_tiles)) {
+        rc = VPZ_E_NOMEM;
+        break;
+      }
+      size_t at = 0;
+      for (const auto& v : task_tiles) {
+        if (!v.empty()) memcpy(ht.p + at, v.data(), v.size() * sizeof(VpzPlaceTile));
+        at += v.size();
+      }
+      ht.n = n_tiles;
+    }
     tt1 = now(); t_deliver += tt1 - tt0; tt0 = tt1;
+    if (dout) {
+      // H2D + K1a + K1b + K3 (unclipped) + K5: the segments and zeros straight into the caller's device buffer
+      if (g.floats > 0) {
+        if (b->total_floats && (rc = batch_decode(b, 0))) break;
+        if ((rc = place_tiles(ctx, slot, b, *dout, clip))) break;
+      }
+      dev::event_record(xb.done[slot], ctx->stream);
+      used[slot] = true;
+      tt1 = now(); t_launch += tt1 - tt0; tt0 = tt1;
+      continue;
+    }
     if (g.floats > 0) {
       if (!xb.d_out[slot].reserve((size_t)g.floats * 4, ctx->last_error) ||
           !xb.d_segs[slot].reserve(std::max<size_t>(n_segs, 1) * sizeof(VpzCopySeg), ctx->last_error)) {
@@ -1495,11 +1669,39 @@ int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const
   if (!rc) rc = r2;
   t_wait += now() - tt0;
   if (trace)
-    fprintf(stderr, "vpz_decode_excerpts: %u excerpts, %zu tasks, %zu groups: files %.1f tasks %.1f plan %.1f commit %.1f replay %.1f launch %.1f wait %.1f ms\n",
-            n, tasks.size(), groups.size(), t_files, t_tasks, t_plan, t_commit, t_deliver, t_launch, t_wait);
+    fprintf(stderr, "vpz_decode_excerpts%s: %u excerpts, %zu tasks, %zu groups: files %.1f tasks %.1f plan %.1f commit %.1f replay %.1f launch %.1f wait %.1f ms\n",
+            dout ? "_device" : "", n, tasks.size(), groups.size(), t_files, t_tasks, t_plan, t_commit, t_deliver, t_launch, t_wait);
   for (int s2 = 0; s2 < 2; s2++)
     if (ctx->bulk[s2]) vpz_batch_reset(ctx->bulk[s2]);
   return rc ? rc : total;
+}
+
+extern "C" {
+
+int64_t vpz_decode_excerpts(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens, uint32_t n,
+                            const uint32_t* file_of, const int64_t* start, const int32_t* count, int clip, float* dst,
+                            size_t dst_floats, int64_t* dst_offsets, int32_t* got) {
+  if (!ctx || !datas || !lens || (n && (!file_of || !start || !count))) return VPZ_E_ARGUMENT;
+  VPZ_USE(ctx);
+  return decode_excerpts_impl(ctx, n_files, datas, lens, n, file_of, start, count, clip, dst, dst_floats, dst_offsets,
+                              got, nullptr);
+}
+
+int64_t vpz_decode_excerpts_device(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
+                                   uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
+                                   int clip, int format, void* dst_dev, size_t dst_elems, int64_t* dst_offsets,
+                                   int32_t* got, void* stream) {
+  if (!ctx || !datas || !lens || (n && (!file_of || !start || !count))) return VPZ_E_ARGUMENT;
+  VPZ_USE(ctx);
+  DevOut o;
+  o.p = dst_dev;
+  o.format = format;
+  o.stream = stream;
+  dev::Event* ev = nullptr;
+  int rc = device_output_begin(ctx, o, &ev);
+  if (rc) return device_output_end(ctx, ev, rc);
+  return device_output_end(ctx, ev, decode_excerpts_impl(ctx, n_files, datas, lens, n, file_of, start, count, clip,
+                                                         static_cast<float*>(dst_dev), dst_elems, dst_offsets, got, &o));
 }
 
 // Debug / tests: the page-end granule index of one container image (first logical stream), built on the device
@@ -1530,3 +1732,9 @@ int64_t vpz_debug_page_end_granules(vpz_ctx* ctx, const uint8_t* data, size_t le
 }
 
 }  // extern "C"
+
+#ifdef VPZ_EMU
+// The emulated CPU test build (tests/emu, never linked into libvpz.so) takes the K5 launcher and the caller-memory
+// hooks of the device-output calls above from here.
+#include "../../tests/emu/dev_emu_place.h"
+#endif

@@ -74,6 +74,7 @@ void vpz_ctx_destroy(vpz_ctx* c) {
     dev::event_destroy(c->bulk_ready[i]);
   }
   delete c->xb;
+  delete c->place;
   delete c->pool;
   c->pool = nullptr;
   scan_bufs_destroy(c->scan);
@@ -146,6 +147,9 @@ int vpz_ctx_set(vpz_ctx* c, const char* key, int value) {
   } else if (!strcmp(key, "bulk_threads")) {
     if (value < 0 || value > 256) return VPZ_E_ARGUMENT;
     c->bulk_threads = value;
+  } else if (!strcmp(key, "bulk_threads_device")) {
+    if (value < 0 || value > 256) return VPZ_E_ARGUMENT;
+    c->bulk_threads_device = value;
   } else if (!strcmp(key, "host_threads")) {
     if (value < 0 || value > 256 || c->pool) return VPZ_E_ARGUMENT;  // before the first bulk call
     c->host_threads = value;

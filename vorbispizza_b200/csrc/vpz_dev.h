@@ -240,3 +240,15 @@ struct VpzCopySeg {
   uint32_t n;               // floats
   uint32_t pad;
 };
+
+// ---- K5: placement into the caller's device buffer (k5_place.cuh) -------------------------------------------
+#define VPZ_TILE_SAMPLES 2048                  // samples per tile at most
+#define VPZ_TILE_ZERO 0xffffffffffffffffull    // VpzPlaceTile.src of a tile of zeros
+struct VpzPlaceTile {
+  uint64_t src;             // float offset of the tile's first sample frame in the batch PCM, or VPZ_TILE_ZERO
+  uint64_t base;            // element offset of the item in the destination
+  uint64_t len;             // samples per channel of the item (channel stride of the planar layout)
+  uint64_t first;           // first sample of the tile in the item
+  uint32_t n;               // samples
+  uint32_t ch;              // channels
+};
