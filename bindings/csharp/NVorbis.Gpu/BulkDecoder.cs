@@ -166,6 +166,60 @@ namespace NVorbis.Gpu
             }
         }
 
+        /// <summary>DecodeFilesToDevice with every file converted on the GPU to sampleRate (0: each keeps its own; else
+        /// 1,000..384,000 Hz, torchaudio.functional.resample's default filter) and channels (0: keep, 1: mean, 2: mono
+        /// duplicated, stereo kept).  dstDevice == IntPtr.Zero: only the layout is computed.  sampleCounts receives the
+        /// output samples per channel of each file, offsets the element offset of each file.  Returns the total
+        /// elements of the layout.</summary>
+        public static long DecodeFilesToDevice(GpuContext gpu, ReadOnlyMemory<byte>[] files, int sampleRate, int channels,
+                                               IntPtr dstDevice, long dstElements, out long[] sampleCounts, out long[] offsets,
+                                               bool planar = true, bool int16 = false, bool clip = true, IntPtr stream = default)
+        {
+            using PinnedImages im = new(files);
+            sampleCounts = new long[Math.Max(files.Length, 1)];
+            offsets = new long[Math.Max(files.Length, 1)];
+            VpzOutConv conv = new() { Format = (planar ? Vpz.OutPlanar : 0) | (int16 ? Vpz.OutS16 : 0), SampleRate = sampleRate, Channels = channels };
+            fixed (IntPtr* p = im.Ptrs)
+            fixed (nuint* l = im.Lens)
+            fixed (long* c = sampleCounts, o = offsets)
+            {
+                long rc = Vpz.vpz_decode_files_device_conv(gpu.Handle, (uint)files.Length, (byte**)p, l, clip ? 1 : 0, &conv, dstDevice,
+                                                           (nuint)dstElements, c, o, stream);
+                Vpz.Check(rc, gpu.Handle);
+                return rc;
+            }
+        }
+
+        /// <summary>ReadExcerptsToDevice with every excerpt converted as DecodeFilesToDevice(.., sampleRate, channels, ..)
+        /// converts files; start and count are samples at the output rate, got counts output samples.  Excerpts of one
+        /// count then make a dense [n][channels][count] batch (planar) whatever the rates and layouts of the files.</summary>
+        public static long ReadExcerptsToDevice(GpuContext gpu, ReadOnlyMemory<byte>[] files, (int file, long start, int count)[] excerpts,
+                                                int sampleRate, int channels, IntPtr dstDevice, long dstElements, out long[] offsets,
+                                                out int[] got, bool planar = true, bool int16 = false, bool clip = true,
+                                                IntPtr stream = default)
+        {
+            using PinnedImages im = new(files);
+            int n = excerpts.Length;
+            uint[] fileOf = new uint[Math.Max(n, 1)];
+            long[] start = new long[Math.Max(n, 1)];
+            int[] count = new int[Math.Max(n, 1)];
+            for (int i = 0; i < n; i++) (fileOf[i], start[i], count[i]) = ((uint)excerpts[i].file, excerpts[i].start, excerpts[i].count);
+            offsets = new long[Math.Max(n, 1)];
+            got = new int[Math.Max(n, 1)];
+            VpzOutConv conv = new() { Format = (planar ? Vpz.OutPlanar : 0) | (int16 ? Vpz.OutS16 : 0), SampleRate = sampleRate, Channels = channels };
+            fixed (IntPtr* p = im.Ptrs)
+            fixed (nuint* l = im.Lens)
+            fixed (uint* f = fileOf)
+            fixed (long* s = start, o = offsets)
+            fixed (int* c = count, g = got)
+            {
+                long rc = Vpz.vpz_decode_excerpts_device_conv(gpu.Handle, (uint)files.Length, (byte**)p, l, (uint)n, f, s, c, clip ? 1 : 0,
+                                                              &conv, dstDevice, (nuint)dstElements, o, g, stream);
+                Vpz.Check(rc, gpu.Handle);
+                return rc;
+            }
+        }
+
         /// <summary>The physical Ogg layer of many images on the GPU (PageReaderBase.ReadNextPage / VerifyPage,
         /// Ogg/PageReaderBase.cs:41-84,286-361; Crc.cs:20-63): the valid pages of every image.</summary>
         public static VpzPageInfo[][] ScanPages(GpuContext gpu, ReadOnlyMemory<byte>[] files, out ulong[] wasteBits, out uint[] crcFailures)

@@ -14,6 +14,12 @@ namespace NVorbis.Gpu
     }
 
     [StructLayout(LayoutKind.Sequential)]
+    internal struct VpzOutConv      // vpz_out_conv
+    {
+        public int Format, SampleRate, Channels;
+    }
+
+    [StructLayout(LayoutKind.Sequential)]
     public struct VpzPageInfo       // vpz_page_info, 32 bytes
     {
         public uint Offset, BodyLength, GranuleLo, GranuleHi, Serial, Sequence;
@@ -138,6 +144,9 @@ namespace NVorbis.Gpu
         internal const int OutS16 = 1, OutPlanar = 2;
         [LibraryImport(Lib)] internal static partial long vpz_decode_files_device(IntPtr ctx, uint n, byte** datas, nuint* lens, int clip, int format, IntPtr dstDev, nuint dstElems, long* sampleCounts, IntPtr stream);
         [LibraryImport(Lib)] internal static partial long vpz_decode_excerpts_device(IntPtr ctx, uint nFiles, byte** datas, nuint* lens, uint n, uint* fileOf, long* start, int* count, int clip, int format, IntPtr dstDev, nuint dstElems, long* dstOffsets, int* got, IntPtr stream);
+        // the same with every item converted to conv->SampleRate / conv->Channels (0: keep) on the GPU (K6)
+        [LibraryImport(Lib)] internal static partial long vpz_decode_files_device_conv(IntPtr ctx, uint n, byte** datas, nuint* lens, int clip, VpzOutConv* conv, IntPtr dstDev, nuint dstElems, long* sampleCounts, long* dstOffsets, IntPtr stream);
+        [LibraryImport(Lib)] internal static partial long vpz_decode_excerpts_device_conv(IntPtr ctx, uint nFiles, byte** datas, nuint* lens, uint n, uint* fileOf, long* start, int* count, int clip, VpzOutConv* conv, IntPtr dstDev, nuint dstElems, long* dstOffsets, int* got, IntPtr stream);
         [LibraryImport(Lib)] internal static partial long vpz_debug_page_end_granules(IntPtr ctx, byte* data, nuint len, int onDevice, long* dst, nuint cap);
     }
 }

@@ -342,6 +342,45 @@ int64_t vpz_decode_excerpts_device(vpz_ctx* ctx, uint32_t n_files, const uint8_t
                                    int clip, int format, void* dst_dev, size_t dst_elems,
                                    int64_t* dst_offsets, int32_t* got, void* stream);
 
+/* ---- the same with conversion to one sample rate and channel layout ------------------------------------------ */
+typedef struct {
+  int32_t format;       /* VPZ_OUT_* bits, as for the *_device calls */
+  int32_t sample_rate;  /* 0: every stream keeps its rate; else 1,000..384,000 Hz: every item is converted to it */
+  int32_t channels;     /* 0: keep; 1: mono = mean of the stream's channels; 2: mono duplicated, stereo kept
+                           (more than 2 source channels: VPZ_E_UNSUPPORTED) */
+} vpz_out_conv;
+
+/* vpz_decode_files_device / vpz_decode_excerpts_device with every item converted to conv->sample_rate and
+ * conv->channels on the device (K6), in the same last pass over the decoded PCM.  Pointer, stream and size checks,
+ * the size query, the format bits and the errors are those of the *_device calls; a sample_rate outside
+ * 1,000..384,000 (other than 0) or channels outside {0, 1, 2} fail with VPZ_E_ARGUMENT.
+ *   Unconverted items (rate 0 or the stream's own, channels 0 or the stream's own) are bitwise what the *_device
+ *   call writes.  Mono is the sum of the channels in channel order divided by C (fp32, round to nearest); at equal
+ *   rates that is the output.  Rate conversion is torchaudio.functional.resample's default (sinc_interp_hann,
+ *   lowpass_filter_width W = 6, rolloff 0.99) in closed form, fi -> fo, base = 0.99 * min(fi, fo):
+ *     y[j] = (base / fi) * sum_k x[k] sinc(t) cos^2(pi t / 2W),  t = clamp(base (k / fi - j / fo), -W, W)
+ *   with x[k] = 0 outside the delivered samples; with o / n = fi / fo in lowest terms only the 2 width + 2 taps
+ *   k in [floor(j o / n) - width, floor(j o / n) + width + 1] can be nonzero, width = ceil(6 o / (0.99 min(o, n))).
+ *   ClipSamples applies to the decoded samples, before mixing and the filter; fp32 output is not clipped again,
+ *   int16 clamps.  A rate pair whose coefficient table exceeds 2^22 floats fails with VPZ_E_UNSUPPORTED.
+ * Files: sample_counts[k] = ceil(n_k fo / fi) for a converted file (n_k: vpz_decode_files' count), dst_offsets
+ *   (may be NULL) the prefix sums of sample_counts * C_out (C_out = conv->channels, or the stream's when 0).  The
+ *   filter sees zeros outside the file.
+ * Excerpts: start / count are output-rate samples.  A converted item reads the source window k_lo =
+ *   max(0, floor(start o / n) - width), k_hi = floor((start + count - 1) o / n) + width + 1 exactly as the plain call
+ *   reads (k_lo, k_hi - k_lo) (width 0 at equal rates); with d samples delivered and e = k_lo + d,
+ *   got = clamp(ceil(e n / o) - start, 0, count), or the negative SeekTo status.  Output samples from got on are
+ *   zero.  A source window longer than the plain call takes as a count (INT32_MAX / 8 samples), or a start past
+ *   2^40 samples, fails with VPZ_E_ARGUMENT.
+ * channels = 2 with a source of more than 2 channels fails with VPZ_E_UNSUPPORTED before anything is decoded. */
+int64_t vpz_decode_files_device_conv(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens,
+                                     int clip, const vpz_out_conv* conv, void* dst_dev, size_t dst_elems,
+                                     int64_t* sample_counts, int64_t* dst_offsets, void* stream);
+int64_t vpz_decode_excerpts_device_conv(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
+                                        uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
+                                        int clip, const vpz_out_conv* conv, void* dst_dev, size_t dst_elems,
+                                        int64_t* dst_offsets, int32_t* got, void* stream);
+
 /* Debug / tests: the page-end granule index SeekTo searches in (PacketProvider.FillPageEndGranuleCache,
  * Ogg/PacketProvider.cs:203-307) of one container image's first logical stream: entry p = granules up to and
  * including page p.  on_device 1: built by the GPU (page scan + one warp per file over its pages), VPZ_E_UNSUPPORTED

@@ -38,6 +38,10 @@ class SetupInfo(C.Structure):
                 ("max_codeword_bits", C.c_int32), ("table_bytes", C.c_uint64)]
 
 
+class OutConv(C.Structure):   # vpz_out_conv
+    _fields_ = [("format", C.c_int32), ("sample_rate", C.c_int32), ("channels", C.c_int32)]
+
+
 class PacketDump(C.Structure):
     _fields_ = [("status", C.c_int32), ("mode", C.c_int32), ("block_size", C.c_int32), ("info", C.c_int32 * 6),
                 ("bits_read", C.c_int32), ("exec_mask", C.c_int32), ("no_execute_mask", C.c_int32),
@@ -126,6 +130,10 @@ _SIGS = {
     "vpz_decode_files_device": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_int, C.c_int, _P, C.c_size_t, _P, _P]),
     "vpz_decode_excerpts_device": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_uint32, _P, _P, _P, C.c_int, C.c_int, _P,
                                                C.c_size_t, _P, _P, _P]),
+    "vpz_decode_files_device_conv": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_int, C.POINTER(OutConv), _P, C.c_size_t,
+                                                 _P, _P, _P]),
+    "vpz_decode_excerpts_device_conv": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_uint32, _P, _P, _P, C.c_int,
+                                                    C.POINTER(OutConv), _P, C.c_size_t, _P, _P, _P]),
     "vpz_debug_page_end_granules":(C.c_int64, [_P, _P, C.c_size_t, C.c_int, _P, C.c_size_t]),
     "vpz_scan_pages": (C.c_int64, [_P, C.c_uint32, _P, _P, _P, C.c_size_t, _P, _P, _P, _P]),
 }

@@ -523,7 +523,15 @@ def _vorbis_channels(data):
     return data[i + 11] if i >= 0 and i + 11 < len(data) else 0
 
 
-def decode_files_device(ctx, files, clip=True, dtype="float32", planar=True, out=None, stream=None):
+def _conv(fmt, sample_rate, channels):
+    """The vpz_out_conv of sample_rate / channels keywords, or None when neither is given (the plain *_device call)."""
+    if sample_rate is None and channels is None:
+        return None
+    return N.OutConv(fmt, int(sample_rate or 0), int(channels or 0))
+
+
+def decode_files_device(ctx, files, clip=True, dtype="float32", planar=True, out=None, stream=None, sample_rate=None,
+                        channels=None):
     """vpz_decode_files_device: decode_files with the PCM left in device memory.
 
     Returns (buf, offsets, counts): buf is one flat buffer of `dtype` ("float32", or "int16" by the reference
@@ -531,13 +539,28 @@ def decode_files_device(ctx, files, clip=True, dtype="float32", planar=True, out
     channel-major [C_k][counts[k]] with planar=True, interleaved otherwise.  When every file has the same channel
     count C and length T, ``buf.view(n, C, T)`` is the batch.  out: a caller tensor (contiguous, on the context's
     device) instead of a new one; stream: the torch / CUDA stream the result is used on (default: the current one);
-    the call waits for the work queued on it and returns when buf is complete."""
+    the call waits for the work queued on it and returns when buf is complete.
+
+    sample_rate / channels (vpz_decode_files_device_conv): every file converted on the GPU to that rate
+    (torchaudio.functional.resample's default filter) and to 1 channel (the mean) or 2 (mono duplicated); None or 0
+    keeps the stream's own.  counts are then output samples and offsets the converted layout's."""
     keep = [_u8(f) for f in files]
     n = len(keep)
     ptrs = (C.c_void_p * n)(*[k[1] for k in keep])
     lens = (C.c_size_t * n)(*[k[2] for k in keep])
     counts = np.zeros(n, np.int64)
     fmt = _format(dtype, planar)
+    conv = _conv(fmt, sample_rate, channels)
+    if conv is not None:
+        offsets = np.zeros(n, np.int64)
+        args = (ctx._h, n, ptrs, lens, int(bool(clip)), C.byref(conv))
+        total = None
+        if out is None:
+            total = ctx.check(ctx.lib.vpz_decode_files_device_conv(*args, None, 0, counts.ctypes.data, None, None))
+        buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
+        total = ctx.check(ctx.lib.vpz_decode_files_device_conv(*args, ptr, elems, counts.ctypes.data,
+                                                               offsets.ctypes.data, handle))
+        return buf[:total], offsets, counts
     args = (ctx._h, n, ptrs, lens, int(bool(clip)), fmt)
     total = None
     if out is None:
@@ -552,13 +575,17 @@ def decode_files_device(ctx, files, clip=True, dtype="float32", planar=True, out
 
 
 def decode_excerpts_device(ctx, files, file_of, start, count, clip=True, dtype="float32", planar=True, out=None,
-                           stream=None):
+                           stream=None, sample_rate=None, channels=None):
     """vpz_decode_excerpts_device: decode_excerpts with the PCM left in device memory.
 
     Returns (buf, offsets, got) as decode_excerpts does; excerpt i starts at element offsets[i] and holds count[i]
     samples per channel, channel-major with planar=True; samples not delivered are zero.  With one channel count C
     and a uniform count T (a crop batch), ``buf.view(n, C, T)`` is the batch.  dtype, out, stream: as
-    decode_files_device."""
+    decode_files_device.
+
+    sample_rate / channels (vpz_decode_excerpts_device_conv): as decode_files_device; start and count are then
+    samples at the output rate, and got counts output samples.  A mixed-rate, mixed-layout corpus cropped to one
+    rate, channel count and length is one dense [n, C, T] batch."""
     keep = [_u8(f) for f in files]
     nf = len(keep)
     ptrs = (C.c_void_p * nf)(*[k[1] for k in keep])
@@ -569,13 +596,16 @@ def decode_excerpts_device(ctx, files, file_of, start, count, clip=True, dtype="
     n = file_of.size
     offsets = np.zeros(n, np.int64)
     got = np.zeros(n, np.int32)
+    fmt = _format(dtype, planar)
+    conv = _conv(fmt, sample_rate, channels)
+    fn = ctx.lib.vpz_decode_excerpts_device if conv is None else ctx.lib.vpz_decode_excerpts_device_conv
     args = (ctx._h, nf, ptrs, lens, n, file_of.ctypes.data, start.ctypes.data, count.ctypes.data, int(bool(clip)),
-            _format(dtype, planar))
+            fmt if conv is None else C.byref(conv))
     total = None
     if out is None:
-        total = ctx.check(ctx.lib.vpz_decode_excerpts_device(*args, None, 0, offsets.ctypes.data, got.ctypes.data, None))
+        total = ctx.check(fn(*args, None, 0, offsets.ctypes.data, got.ctypes.data, None))
     buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
-    total = ctx.check(ctx.lib.vpz_decode_excerpts_device(*args, ptr, elems, offsets.ctypes.data, got.ctypes.data, handle))
+    total = ctx.check(fn(*args, ptr, elems, offsets.ctypes.data, got.ctypes.data, handle))
     return buf[:total], offsets, got
 
 

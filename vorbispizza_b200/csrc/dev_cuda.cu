@@ -12,6 +12,7 @@
 #include "k3_streams.cuh"
 #include "k4_deliver.cuh"
 #include "k5_place.cuh"
+#include "k6_convert.cuh"
 
 // ---- kernels ---------------------------------------------------------------------------------
 __global__ void __launch_bounds__(K0_THREADS) vpz_k0_pages(K0Params P) {
@@ -30,6 +31,12 @@ __global__ void __launch_bounds__(K4_THREADS) vpz_k4_deliver(K4Params P) { k4_ct
 
 template <bool OUT16, bool PLANAR>
 __global__ void __launch_bounds__(K5_THREADS) vpz_k5_place(K5Params P) { k5_cta<OUT16, PLANAR>(P); }
+
+template <bool OUT16, bool PLANAR>
+__global__ void __launch_bounds__(K6_THREADS) vpz_k6_convert(K6Params P) {
+  extern __shared__ float k6_smem[];
+  k6_cta<OUT16, PLANAR>(P, k6_smem);
+}
 
 #ifndef K1A_MIN_CTAS
 #define K1A_MIN_CTAS 8
@@ -170,6 +177,10 @@ int init(int device, int* resolved, std::string& err) {
   allow_max_smem(vpz_k3_streams<true, false>, optin);
   allow_max_smem(vpz_k3_streams<false, true>, optin);
   allow_max_smem(vpz_k3_streams<true, true>, optin);
+  allow_max_smem(vpz_k6_convert<false, false>, optin);
+  allow_max_smem(vpz_k6_convert<false, true>, optin);
+  allow_max_smem(vpz_k6_convert<true, false>, optin);
+  allow_max_smem(vpz_k6_convert<true, true>, optin);
   e = cudaGetLastError();
   if (e != cudaSuccess) return fail(e, "cudaFuncSetAttribute", err);
   return VPZ_OK;
@@ -319,6 +330,23 @@ int launch_k5(const K5Params& p, Stream* s, std::string& err) {
   }
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k5_place", err);
+}
+
+int launch_k6(const K6Params& p, Stream* s, std::string& err) {
+  if (p.n_tiles == 0) return VPZ_OK;
+  const size_t smem = (size_t)p.smem_floats * 4;
+  if (smem > max_smem_per_block()) {
+    err = "vpz_k6_convert: a tile needs " + std::to_string(smem) + " bytes of shared memory";
+    return VPZ_E_UNSUPPORTED;
+  }
+  const unsigned grid = (unsigned)std::min<size_t>(p.n_tiles, (size_t)8 * sm_count());
+  if (p.out16) {
+    if (p.planar) vpz_k6_convert<true, true><<<grid, K6_THREADS, smem, s->s>>>(p); else vpz_k6_convert<true, false><<<grid, K6_THREADS, smem, s->s>>>(p);
+  } else {
+    if (p.planar) vpz_k6_convert<false, true><<<grid, K6_THREADS, smem, s->s>>>(p); else vpz_k6_convert<false, false><<<grid, K6_THREADS, smem, s->s>>>(p);
+  }
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k6_convert", err);
 }
 
 int check_device_ptr(const void* p, int device, std::string& err) {

@@ -70,6 +70,9 @@ int launch_k0g(const K0gParams& p, Stream* s, std::string& err);
 int launch_k4(const K4Params& p, Stream* s, std::string& err);
 // K5: tiles of the batch PCM into the caller's device buffer, one warp per tile
 int launch_k5(const K5Params& p, Stream* s, std::string& err);
+// K6: rate / channel conversion of tiles into the caller's device buffer, one CTA per tile, p.smem_floats * 4 bytes of
+// dynamic shared memory (VPZ_E_UNSUPPORTED when that exceeds the device's limit)
+int launch_k6(const K6Params& p, Stream* s, std::string& err);
 
 // Caller-owned device memory (the *_device bulk calls): 0 when p is device or managed memory of `device`,
 // VPZ_E_ARGUMENT (with the reason in err) for host, pinned or another device's memory

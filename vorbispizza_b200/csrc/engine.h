@@ -8,6 +8,7 @@
 #include <condition_variable>
 #include <functional>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -170,9 +171,20 @@ struct ExcerptBufs {
   }
 };
 
+struct ConvFilter {   // K6 coefficient table of one rate pair: 2 width + 2 taps x n phases (tap-major), uploaded once
+  int fi = 0, fo = 0;
+  uint32_t o = 1, n = 1, width = 0;
+  std::vector<float> host;
+  DevBuf dev;
+};
+
 struct PlaceBufs {   // one slot per pipeline batch (vpz_decode_files_device: 3, vpz_decode_excerpts_device: 2)
   HostBuf<VpzPlaceTile> h_tiles[3];
   DevBuf d_tiles[3];
+  HostBuf<VpzConvTile> h_ctiles[3];   // the *_conv calls: K6 tiles
+  DevBuf d_ctiles[3];
+  DevBuf d_scratch[2];                // vpz_decode_excerpts_device_conv: source windows of converted excerpts (K5 -> K6)
+  std::vector<std::unique_ptr<ConvFilter>> filters;   // by rate pair, kept across calls
 };
 
 struct PktSrc {

@@ -79,6 +79,16 @@ struct K5Params {
   int clip;                        // clip before the conversion (the excerpt path decodes unclipped)
 };
 
+struct K6Params {
+  const float* src;                // interleaved fp32 source items: the batch PCM (files) or the slot's scratch (excerpts)
+  void* out;                       // the caller's device buffer: fp32 or int16 elements
+  const VpzConvTile* tiles;
+  uint32_t n_tiles;
+  uint32_t smem_floats;            // shared memory of the largest tile (staged frames x staged channels)
+  int planar;                      // 1: channel-major items, 0: interleaved
+  int out16;                       // 1: int16 elements by K3's rule (k3_s16)
+};
+
 struct K0gParams {
   const uint8_t* images;           // the staged images of the K0 scan
   const VpzGranFile* files;

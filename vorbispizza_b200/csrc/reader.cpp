@@ -22,9 +22,11 @@
 #include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <cmath>
 #include <deque>
 #include <memory>
 #include <new>
+#include <numeric>
 #include <thread>
 
 #include "../../include/vpz.h"
@@ -879,6 +881,8 @@ struct DevOut {
   void* p = nullptr;       // the caller's device buffer (NULL: size query)
   int format = 0;          // VPZ_OUT_* bits
   void* stream = nullptr;  // the caller's cudaStream_t
+  const vpz_out_conv* conv = nullptr;   // the *_conv calls: target rate and channels (K6)
+  int64_t* offsets = nullptr;           // vpz_decode_files_device_conv: element offset of every file (may be NULL)
 };
 
 size_t tile_count(uint64_t samples) { return (size_t)((samples + VPZ_TILE_SAMPLES - 1) / VPZ_TILE_SAMPLES); }
@@ -940,25 +944,236 @@ int64_t device_output_end(vpz_ctx* ctx, dev::Event* ev, int64_t rc) {
   return rc;
 }
 
-// Uploads the tiles of pipeline slot `slot` and launches K5 on the context's stream
-int place_tiles(vpz_ctx* ctx, int slot, const vpz_batch* b, const DevOut& o, int clip) {
+// Uploads the tiles of pipeline slot `slot` and launches K5 on the context's stream.  Tiles [0, n_dst) go to the
+// caller's buffer; the rest (vpz_decode_excerpts_device_conv) to the slot's scratch, as fp32 interleaved.
+int place_tiles(vpz_ctx* ctx, int slot, const vpz_batch* b, const DevOut& o, int clip, size_t n_dst = SIZE_MAX) {
   PlaceBufs& pb = *ctx->place;
   const size_t n = pb.h_tiles[slot].n;
   if (!n) return VPZ_OK;
   if (!pb.d_tiles[slot].reserve(n * sizeof(VpzPlaceTile), ctx->last_error)) return VPZ_E_CUDA;
   int rc = dev::h2d(pb.d_tiles[slot].p, pb.h_tiles[slot].p, n * sizeof(VpzPlaceTile), ctx->stream, ctx->last_error);
   if (rc) return rc;
+  n_dst = std::min(n_dst, n);
   K5Params kp;
   kp.pcm = static_cast<const float*>(b->d_pcm.p);
   kp.out = o.p;
   kp.tiles = static_cast<const VpzPlaceTile*>(pb.d_tiles[slot].p);
-  kp.n_tiles = (uint32_t)n;
+  kp.n_tiles = (uint32_t)n_dst;
   kp.planar = (o.format & VPZ_OUT_PLANAR) ? 1 : 0;
   kp.out16 = (o.format & VPZ_OUT_S16) ? 1 : 0;
   kp.clip = clip ? 1 : 0;
   rc = dev::launch_k5(kp, ctx->stream, ctx->last_error);
+  if (!rc && n_dst) ctx->kernel_launches++;
+  if (rc || n_dst == n) return rc;
+  kp.out = pb.d_scratch[slot].p;
+  kp.tiles += n_dst;
+  kp.n_tiles = (uint32_t)(n - n_dst);
+  kp.planar = 0;
+  kp.out16 = 0;
+  rc = dev::launch_k5(kp, ctx->stream, ctx->last_error);
   if (!rc) ctx->kernel_launches++;
   return rc;
+}
+
+// ---- conversion to one rate and channel layout (the *_conv calls, K6) ------------------------------------------
+int conv_check(vpz_ctx* ctx, const vpz_out_conv* cv) {
+  if (!cv || (cv->sample_rate != 0 && (cv->sample_rate < 1000 || cv->sample_rate > 384000)) || cv->channels < 0 ||
+      cv->channels > 2) {
+    ctx->last_error = cv ? "conversion: sample_rate must be 0 or 1000..384000, channels 0, 1 or 2" : "conversion: NULL";
+    return VPZ_E_ARGUMENT;
+  }
+  return VPZ_OK;
+}
+
+int64_t floor_div(int64_t a, int64_t b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+// What K6 does to the items of one stream (rate fi, C channels)
+struct ItemConv {
+  bool on = false;                 // converted; otherwise K5 places the item unchanged
+  const ConvFilter* f = nullptr;   // the rate pair's table once uploaded (NULL at equal rates and in a size query)
+  bool filter = false;             // rates differ
+  uint32_t o = 1, n = 1, width = 0;
+  uint32_t C = 0, Cout = 0, mix = VPZ_MIX_KEEP;
+  uint32_t m = 0;                  // output samples per tile
+  uint32_t smem_floats = 0;        // shared memory of the largest tile
+  int64_t out_len(int64_t src) const { return filter ? (src * n + o - 1) / o : src; }   // ceil(src fo / fi)
+  // source window [k_lo, k_hi) of output samples [start, start + count)
+  void window(int64_t start, int64_t count, int64_t* k_lo, int64_t* k_hi) const {
+    if (!filter) {
+      *k_lo = start;
+      *k_hi = start + count;
+      return;
+    }
+    *k_lo = std::max<int64_t>(0, floor_div(start * o, n) - width);
+    *k_hi = std::max(*k_lo, floor_div((start + count - 1) * o, n) + width + 1);
+  }
+};
+
+// The coefficient table of fi -> fo, made and uploaded on first use and kept in the context: tap-major, entry
+// [i][p] weighs source frame k = floor(p o / n) - width + i, i < 2 width + 2, of output p (torchaudio.functional.resample's sinc_interp_hann,
+// W = 6, rolloff 0.99, evaluated in float64)
+int conv_filter(vpz_ctx* ctx, int fi, int fo, const ConvFilter** out) {
+  PlaceBufs& pb = *ctx->place;
+  for (const auto& f : pb.filters)
+    if (f->fi == fi && f->fo == fo) {
+      *out = f.get();
+      return VPZ_OK;
+    }
+  std::unique_ptr<ConvFilter> f(new (std::nothrow) ConvFilter);
+  if (!f) return VPZ_E_NOMEM;
+  const uint32_t g = (uint32_t)std::gcd(fi, fo);
+  f->fi = fi;
+  f->fo = fo;
+  f->o = (uint32_t)fi / g;
+  f->n = (uint32_t)fo / g;
+  const double W = 6.0, base = 0.99 * std::min(f->o, f->n), pi = 3.14159265358979323846;
+  f->width = (uint32_t)std::ceil(W * f->o / base);
+  const uint32_t taps = 2 * f->width + 2;
+  f->host.resize((size_t)f->n * taps);
+  for (uint32_t p = 0; p < f->n; p++) {
+    const int64_t k0 = (int64_t)p * f->o / f->n - f->width;
+    for (uint32_t i = 0; i < taps; i++) {
+      double t = base * ((double)(k0 + i) / f->o - (double)p / f->n);
+      t = std::min(W, std::max(-W, t));
+      const double w = std::cos(t * pi / (2 * W));
+      const double sinc = t == 0 ? 1.0 : std::sin(pi * t) / (pi * t);
+      f->host[(size_t)i * f->n + p] = (float)(base / f->o * sinc * w * w);
+    }
+  }
+  if (!f->dev.reserve(f->host.size() * 4, ctx->last_error)) return VPZ_E_CUDA;
+  int rc = dev::h2d(f->dev.p, f->host.data(), f->host.size() * 4, ctx->stream, ctx->last_error);
+  if (rc) return rc;
+  *out = f.get();
+  pb.filters.push_back(std::move(f));
+  return VPZ_OK;
+}
+
+// Plans the items of a stream (rate fi, C channels); build: also fetch the table (the call writes samples)
+int conv_plan(vpz_ctx* ctx, const vpz_out_conv& cv, int fi, int C, bool build, ItemConv* ic) {
+  *ic = ItemConv();
+  ic->C = (uint32_t)C;
+  ic->Cout = cv.channels ? (uint32_t)cv.channels : (uint32_t)C;
+  if (C > 2 && cv.channels == 2) {
+    ctx->last_error = "conversion: channels = 2 from a stream of more than 2 channels";
+    return VPZ_E_UNSUPPORTED;
+  }
+  const int fo = cv.sample_rate ? cv.sample_rate : fi;
+  ic->mix = ic->Cout == ic->C ? VPZ_MIX_KEEP : ic->Cout == 1 ? VPZ_MIX_MEAN : VPZ_MIX_DUP;
+  ic->filter = fo != fi;
+  ic->on = ic->filter || ic->mix != VPZ_MIX_KEEP;
+  if (!ic->on) return VPZ_OK;
+  if (ic->filter) {
+    if (fi <= 0) {
+      ctx->last_error = "conversion: stream without a sample rate";
+      return VPZ_E_UNSUPPORTED;
+    }
+    const uint32_t g = (uint32_t)std::gcd(fi, fo);
+    ic->o = (uint32_t)fi / g;
+    ic->n = (uint32_t)fo / g;
+    ic->width = (uint32_t)std::ceil(6.0 * ic->o / (0.99 * std::min(ic->o, ic->n)));
+    if ((uint64_t)ic->n * (2 * ic->width + 2) > K6_MAX_TAB_FLOATS) {
+      ctx->last_error = "conversion: the coefficient table of " + std::to_string(fi) + " -> " + std::to_string(fo) +
+                        " Hz exceeds 2^22 floats";
+      return VPZ_E_UNSUPPORTED;
+    }
+    if (build) {
+      int rc = conv_filter(ctx, fi, fo, &ic->f);
+      if (rc) return rc;
+    }
+  }
+  // tile size: the staged span (frames x staged floats per frame) within K6_SMEM_BUDGET where one output allows it
+  const uint32_t per_frame = ic->mix == VPZ_MIX_MEAN ? ic->C + 1 : ic->C;
+  const uint64_t budget = K6_SMEM_BUDGET / 4 / per_frame;
+  auto span = [&](uint64_t m) { return ic->filter ? ((ic->n - 1) + (m - 1) * ic->o) / ic->n + 2 * ic->width + 2 : m; };
+  uint64_t m = K6_MAX_OUTS;
+  if (ic->filter) {
+    const uint64_t fixed = 2 * ic->width + 3;
+    m = budget > fixed ? std::min<uint64_t>(m, (budget - fixed) * ic->n / ic->o + 1) : 1;
+  } else {
+    m = std::min<uint64_t>(m, budget);
+  }
+  while (m > 1 && span(m) > budget) m--;
+  ic->m = (uint32_t)m;
+  ic->smem_floats = (uint32_t)(span(m) * per_frame);
+  return VPZ_OK;
+}
+
+size_t conv_tile_count(const ItemConv& ic, uint64_t len) { return (size_t)((len + ic.m - 1) / ic.m); }
+
+// K6 tiles of one item: `len` output samples (element base `base`), output sample 0 is j = j_first of the stream;
+// its source is `src_len` frames at float offset src, source frame 0 is k = k_first; outputs from `valid` on are zero
+VpzConvTile* put_conv_tiles(VpzConvTile* out, const ItemConv& ic, uint64_t src, int64_t k_first, uint64_t src_len,
+                            uint64_t base, uint64_t len, int64_t j_first, uint64_t valid) {
+  for (uint64_t s = 0; s < len; s += ic.m) {
+    VpzConvTile t;
+    memset(&t, 0, sizeof(t));
+    const uint32_t n = (uint32_t)std::min<uint64_t>(ic.m, len - s);
+    const int64_t j0 = j_first + (int64_t)s;
+    t.src = src;
+    t.base = base;
+    t.len = len;
+    t.first = s;
+    t.n = n;
+    t.valid = valid > s ? (uint32_t)std::min<uint64_t>(valid - s, n) : 0;
+    t.src_len = (uint32_t)src_len;
+    t.ch_src = (uint8_t)ic.C;
+    t.ch_out = (uint8_t)ic.Cout;
+    t.mix = (uint8_t)ic.mix;
+    if (ic.filter) {
+      const int64_t a = j0 * ic.o;
+      t.taps = ic.f->dev.p ? static_cast<const float*>(ic.f->dev.p) : nullptr;
+      t.ro = ic.o;
+      t.rn = ic.n;
+      t.width = ic.width;
+      t.p0 = (uint32_t)(j0 % ic.n);
+      t.r0 = (uint32_t)(a % ic.n);
+      t.s_first = a / ic.n - ic.width - k_first;
+      t.span = (t.r0 + (n - 1) * ic.o) / ic.n + 2 * ic.width + 2;
+    } else {
+      t.ro = t.rn = 1;
+      t.s_first = j0 - k_first;
+      t.span = n;
+    }
+    *out++ = t;
+  }
+  return out;
+}
+
+// Uploads the K6 tiles of slot `slot` and launches K6 from src into the caller's buffer
+int convert_tiles(vpz_ctx* ctx, int slot, const void* src, const DevOut& o) {
+  PlaceBufs& pb = *ctx->place;
+  const size_t n = pb.h_ctiles[slot].n;
+  if (!n) return VPZ_OK;
+  uint32_t smem = 0;
+  for (size_t i = 0; i < n; i++) {
+    const VpzConvTile& t = pb.h_ctiles[slot].p[i];
+    smem = std::max<uint32_t>(smem, t.span * (t.ch_src + (t.mix == VPZ_MIX_MEAN ? 1u : 0u)));
+  }
+  if (!pb.d_ctiles[slot].reserve(n * sizeof(VpzConvTile), ctx->last_error)) return VPZ_E_CUDA;
+  int rc = dev::h2d(pb.d_ctiles[slot].p, pb.h_ctiles[slot].p, n * sizeof(VpzConvTile), ctx->stream, ctx->last_error);
+  if (rc) return rc;
+  K6Params kp;
+  kp.src = static_cast<const float*>(src);
+  kp.out = o.p;
+  kp.tiles = static_cast<const VpzConvTile*>(pb.d_ctiles[slot].p);
+  kp.n_tiles = (uint32_t)n;
+  kp.smem_floats = smem;
+  kp.planar = (o.format & VPZ_OUT_PLANAR) ? 1 : 0;
+  kp.out16 = (o.format & VPZ_OUT_S16) ? 1 : 0;
+  rc = dev::launch_k6(kp, ctx->stream, ctx->last_error);
+  if (!rc) ctx->kernel_launches++;
+  return rc;
+}
+
+// Channels and rate from the identification header on the first page of a container image (0, 0 when it is not
+// where a well-formed file has it: the decode reports that file's error)
+void peek_id_header(const uint8_t* d, size_t len, int* channels, int* rate) {
+  *channels = *rate = 0;
+  if (!d || len < 27 || memcmp(d, "OggS", 4)) return;
+  const size_t body = 27 + (size_t)d[26];
+  if (body + 16 > len || memcmp(d + body, "\x01vorbis", 7)) return;
+  *channels = d[body + 11];
+  *rate = (int)((uint32_t)d[body + 12] | (uint32_t)d[body + 13] << 8 | (uint32_t)d[body + 14] << 16 | (uint32_t)d[body + 15] << 24);
 }
 }  // namespace
 
@@ -1073,7 +1288,8 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
     t1 = now(); t_plan += t1 - t0; t0 = t1;
     std::vector<RunPlan*> plans;
     plans.reserve(cnt);
-    uint64_t group_floats = 0;
+    uint64_t group_floats = 0, group_out = 0;   // batch PCM floats; elements of the destination
+    std::vector<ItemConv> conv(dout && dout->conv ? cnt : 0);
     for (uint32_t i = 0; i < cnt; i++) {
       BulkJob& j = *jobs[i];
       if (j.rc) {
@@ -1081,17 +1297,25 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
         ctx->last_error = j.err;
         break;
       }
-      int64_t samples = j.win.has_plan ? j.win.plan.samples : 0;
-      if (sample_counts) sample_counts[first + i] = samples;
+      int64_t samples = j.win.has_plan ? j.win.plan.samples : 0, out = samples;
+      uint32_t ch = (uint32_t)j.dec.channels();
+      if (!conv.empty()) {
+        if ((rc = conv_plan(ctx, *dout->conv, j.dec.setup->host.id.sample_rate, (int)ch, dst != nullptr, &conv[i]))) break;
+        out = conv[i].out_len(samples);
+        ch = conv[i].Cout;
+        if (dout->offsets) dout->offsets[first + i] = total + (int64_t)group_out;
+      }
+      if (sample_counts) sample_counts[first + i] = out;
       group_floats += (uint64_t)samples * j.dec.channels();
+      group_out += (uint64_t)out * ch;
       if (j.win.has_plan) plans.push_back(&j.win.plan);
     }
     if (rc) break;
     if (!dst) {  // size query: nothing is decoded
-      total += (int64_t)group_floats;
+      total += (int64_t)group_out;
       continue;
     }
-    if ((uint64_t)total + group_floats > dst_floats) {
+    if ((uint64_t)total + group_out > dst_floats) {
       ctx->last_error = "destination buffer too small";
       rc = VPZ_E_ARGUMENT;
       break;
@@ -1116,25 +1340,36 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
     }
     if (dout && group_floats) {
       // 4b. K5 tiles: file i of the group is the batch PCM at its offset in the group (runs are committed in
-      //     file order), placed at element total + that offset
-      std::vector<uint64_t> off(cnt + 1, 0);
-      std::vector<size_t> first_tile(cnt + 1, 0);
+      //     file order), placed at element total + that offset.  The _conv call: a converted file gets K6 tiles
+      //     instead, placed at its offset in the converted layout (oo).
+      std::vector<uint64_t> off(cnt + 1, 0), oo(cnt + 1, 0);
+      std::vector<size_t> first_tile(cnt + 1, 0), first_ctile(cnt + 1, 0);
       for (uint32_t i = 0; i < cnt; i++) {
         const BulkJob& j = *jobs[i];
         const int64_t samples = j.win.has_plan ? j.win.plan.samples : 0;
+        const bool on = !conv.empty() && conv[i].on;
         off[i + 1] = off[i] + (uint64_t)samples * j.dec.channels();
-        first_tile[i + 1] = first_tile[i] + tile_count((uint64_t)samples);
+        oo[i + 1] = oo[i] + (on ? (uint64_t)conv[i].out_len(samples) * conv[i].Cout : (uint64_t)samples * j.dec.channels());
+        first_tile[i + 1] = first_tile[i] + (on ? 0 : tile_count((uint64_t)samples));
+        first_ctile[i + 1] = first_ctile[i] + (on ? conv_tile_count(conv[i], (uint64_t)conv[i].out_len(samples)) : 0);
       }
       HostBuf<VpzPlaceTile>& ht = ctx->place->h_tiles[slot];
-      if (!ht.reserve(first_tile[cnt])) {
+      HostBuf<VpzConvTile>& hc = ctx->place->h_ctiles[slot];
+      if (!ht.reserve(first_tile[cnt]) || !hc.reserve(first_ctile[cnt])) {
         rc = VPZ_E_NOMEM;
         break;
       }
       ht.n = first_tile[cnt];
+      hc.n = first_ctile[cnt];
       pool->parallel_for(cnt, [&](size_t i) {
         const BulkJob& j = *jobs[i];
         const uint64_t samples = j.win.has_plan ? (uint64_t)j.win.plan.samples : 0;
-        put_tiles(ht.p + first_tile[i], off[i], (uint64_t)total + off[i], samples, 0, samples, (uint32_t)j.dec.channels());
+        if (!conv.empty() && conv[i].on) {
+          const uint64_t out = (uint64_t)conv[i].out_len((int64_t)samples);
+          put_conv_tiles(hc.p + first_ctile[i], conv[i], off[i], 0, samples, (uint64_t)total + oo[i], out, 0, out);
+        } else {
+          put_tiles(ht.p + first_tile[i], off[i], (uint64_t)total + oo[i], samples, 0, samples, (uint32_t)j.dec.channels());
+        }
       });
     }
     t1 = now(); t_commit += t1 - t0; t0 = t1;
@@ -1142,6 +1377,7 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
       // 5. H2D + K1 + K3 + K5 (batch PCM -> the caller's device buffer) on the compute stream
       if ((rc = batch_decode(b, clip, 0))) break;
       if ((rc = place_tiles(ctx, slot, b, *dout, 0))) break;   // (K3 has clipped)
+      if (dout->conv && (rc = convert_tiles(ctx, slot, b->d_pcm.p, *dout))) break;
     } else if (group_floats) {
       // 5. H2D + K1 + K3 on the compute stream, then the PCM of this group on the copy stream
       if ((rc = batch_decode(b, clip, out16))) break;
@@ -1156,7 +1392,7 @@ static int64_t decode_files_impl(vpz_ctx* ctx, uint32_t n, const uint8_t* const*
     dev::event_record(ctx->bulk_done[slot], dout ? ctx->stream : ctx->copy_stream);
     t1 = now(); t_launch += t1 - t0; t0 = t1;
     used[slot] = true;
-    total += (int64_t)group_floats;
+    total += (int64_t)group_out;
   }
   // drain the pipeline (also on errors: buffers must not be in flight when the jobs are freed)
   for (int s = 0; s < 3; s++)
@@ -1201,6 +1437,33 @@ int64_t vpz_decode_files_device(vpz_ctx* ctx, uint32_t n, const uint8_t* const* 
   o.stream = stream;
   dev::Event* ev = nullptr;
   int rc = device_output_begin(ctx, o, &ev);
+  if (rc) return device_output_end(ctx, ev, rc);
+  return device_output_end(ctx, ev, decode_files_impl(ctx, n, datas, lens, clip, static_cast<float*>(dst_dev), dst_elems,
+                                                      sample_counts, 0, &o));
+}
+
+int64_t vpz_decode_files_device_conv(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int clip,
+                                     const vpz_out_conv* conv, void* dst_dev, size_t dst_elems, int64_t* sample_counts,
+                                     int64_t* dst_offsets, void* stream) {
+  if (!ctx || (n && (!datas || !lens))) return VPZ_E_ARGUMENT;
+  VPZ_USE(ctx);
+  int rc = conv_check(ctx, conv);
+  if (rc) return rc;
+  // streams the conversion refuses fail the call before anything is decoded
+  for (uint32_t i = 0; i < n; i++) {
+    int ch, rate;
+    peek_id_header(datas[i], lens[i], &ch, &rate);
+    ItemConv ic;
+    if (ch > 0 && rate > 0 && (rc = conv_plan(ctx, *conv, rate, ch, false, &ic))) return rc;
+  }
+  DevOut o;
+  o.p = dst_dev;
+  o.format = conv->format;
+  o.stream = stream;
+  o.conv = conv;
+  o.offsets = dst_offsets;
+  dev::Event* ev = nullptr;
+  rc = device_output_begin(ctx, o, &ev);
   if (rc) return device_output_end(ctx, ev, rc);
   return device_output_end(ctx, ev, decode_files_impl(ctx, n, datas, lens, clip, static_cast<float*>(dst_dev), dst_elems,
                                                       sample_counts, 0, &o));
@@ -1365,13 +1628,53 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
     if (rc) return rc;
   }
   tt1 = now(); t_files = tt1 - tt0; tt0 = tt1;
+  // ---- the _conv call: what K6 does to each file's excerpts, and every converted excerpt's source window, which
+  //      the rest of the call decodes as the plain call decodes an excerpt (start / count below are the windows)
+  const vpz_out_conv* cv = dout ? dout->conv : nullptr;
+  std::vector<ItemConv> fconv(cv ? n_files : 0);
+  const int64_t* ostart = start;   // the caller's excerpts (output samples)
+  const int32_t* ocount = count;
+  std::vector<int64_t> xstart;
+  std::vector<int32_t> xcount;
+  if (cv) {
+    for (uint32_t f = 0; f < n_files; f++) {
+      const StreamDec& m = files[f]->master;
+      int rc = conv_plan(ctx, *cv, m.setup->host.id.sample_rate, m.channels(), dst != nullptr, &fconv[f]);
+      if (rc) return rc;
+    }
+    xstart.resize(n);
+    xcount.resize(n);
+    for (uint32_t i = 0; i < n; i++) {
+      if (file_of[i] >= n_files || start[i] < 0 || count[i] < 0) return VPZ_E_ARGUMENT;
+      const ItemConv& ic = fconv[file_of[i]];
+      int64_t lo = start[i], hi = start[i] + count[i];
+      // (far beyond any stream: start * o stays inside 64 bits)
+      if (ic.on && start[i] > ((int64_t)1 << 40)) {
+        ctx->last_error = "conversion: start out of range";
+        return VPZ_E_ARGUMENT;
+      }
+      if (ic.on) ic.window(start[i], count[i], &lo, &hi);
+      if (hi - lo > INT32_MAX / VPZ_MAX_CH) {
+        ctx->last_error = "conversion: source window too long";
+        return VPZ_E_ARGUMENT;
+      }
+      xstart[i] = lo;
+      xcount[i] = (int32_t)(hi - lo);
+    }
+    start = xstart.data();
+    count = xcount.data();
+  }
+  // elements of excerpt i in the destination
+  auto item_elems = [&](uint32_t i) {
+    return cv ? (int64_t)ocount[i] * fconv[file_of[i]].Cout : (int64_t)count[i] * files[file_of[i]]->master.channels();
+  };
   // ---- layout of the destination -------------------------------------------------------------------
   int64_t total = 0;
   for (uint32_t i = 0; i < n; i++) {
     // (count * channels is handed to Read as an int, like Span<float>.Length in the reference)
     if (file_of[i] >= n_files || start[i] < 0 || count[i] < 0 || count[i] > INT32_MAX / VPZ_MAX_CH) return VPZ_E_ARGUMENT;
     if (dst_offsets) dst_offsets[i] = total;
-    total += (int64_t)count[i] * files[file_of[i]]->master.channels();
+    total += item_elems(i);
   }
   if (!dst) return total;
   if ((uint64_t)total > dst_floats) {
@@ -1389,7 +1692,7 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
     int64_t acc = 0;
     for (uint32_t i = 0; i < n; i++) {
       own_offsets[i] = acc;
-      acc += (int64_t)count[i] * files[file_of[i]]->master.channels();
+      acc += item_elems(i);
     }
     dst_offsets = own_offsets.data();
   }
@@ -1492,7 +1795,9 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
   int rc = VPZ_OK;
   bool used[2] = {false, false};
   std::vector<std::vector<VpzCopySeg>> task_segs;
-  std::vector<std::vector<VpzPlaceTile>> task_tiles;
+  std::vector<std::vector<VpzPlaceTile>> task_tiles, task_xtiles;   // K5 into dst / into the scratch (_conv)
+  std::vector<std::vector<VpzConvTile>> task_ctiles;                 // K6 (_conv)
+  std::vector<uint64_t> xoff(cv ? n : 0);                             // float offset of a converted excerpt's window in the scratch
   for (size_t gi = 0; gi < groups.size() && !rc; gi++) {
     const Group& g = groups[gi];
     const int slot = (int)(gi & 1);
@@ -1536,6 +1841,38 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
     // consumer side, samples untouched: SeekTo's two packets, then Read until `count` samples or the end
     task_segs.assign(g.t1 - g.t0, std::vector<VpzCopySeg>());
     if (dout) task_tiles.assign(g.t1 - g.t0, std::vector<VpzPlaceTile>());
+    uint64_t scratch = 0;
+    if (cv) {
+      task_xtiles.assign(g.t1 - g.t0, std::vector<VpzPlaceTile>());
+      task_ctiles.assign(g.t1 - g.t0, std::vector<VpzConvTile>());
+      for (uint32_t i = g.i0; i < g.i1; i++)
+        if (fconv[file_of[i]].on) {
+          xoff[i] = scratch;
+          scratch += (uint64_t)count[i] * fconv[file_of[i]].C;
+        }
+      if (scratch && !ctx->place->d_scratch[slot].reserve(scratch * 4, ctx->last_error)) {
+        rc = VPZ_E_CUDA;
+        break;
+      }
+    }
+    // a converted excerpt i whose window delivered `have` samples (status: SeekTo's error, or 0): zeros behind them
+    // in the scratch, got by the output rate, K6 tiles from the scratch into dst
+    auto conv_item = [&](size_t k, uint32_t i, int have, int status) {
+      const ItemConv& ic = fconv[file_of[i]];
+      append_tiles(task_xtiles[k], VPZ_TILE_ZERO, xoff[i], count[i], have, count[i] - have, ic.C);
+      int64_t g_out = status;
+      if (!status) {
+        const int64_t e = start[i] + have;   // the window starts at k_lo = start[i]
+        g_out = (ic.filter ? (e * ic.n + ic.o - 1) / ic.o : e) - ostart[i];
+        g_out = std::max<int64_t>(0, std::min<int64_t>(g_out, ocount[i]));
+      }
+      if (got) got[i] = (int32_t)g_out;
+      std::vector<VpzConvTile>& v = task_ctiles[k];
+      const size_t at = v.size();
+      v.resize(at + conv_tile_count(ic, (uint64_t)ocount[i]));
+      put_conv_tiles(v.data() + at, ic, xoff[i], start[i], (uint64_t)count[i], (uint64_t)dst_offsets[i],
+                     (uint64_t)ocount[i], ostart[i], status ? 0 : (uint64_t)g_out);
+    };
     pool->parallel_for(g.t1 - g.t0, [&](size_t k) {
       ExcerptTask& t = tasks[g.t0 + k];
       StreamDec* d = t.dec.get();
@@ -1544,15 +1881,18 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
       for (size_t q = 0; q < t.count; q++) {
         ExcerptJob& j = jobs[t.first + q];
         const uint32_t i = j.index;
+        const bool conv_on = cv && fconv[t.file].on;
         if (j.status) {
           if (got) got[i] = j.status;
-          if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
+          if (conv_on) conv_item(k, i, 0, j.status);
+          else if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
           continue;
         }
         int prc = place_window(d, b, j.win.get(), j.run, j.drain_run, 0);
         if (prc) {
           if (got) got[i] = prc;
-          if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
+          if (conv_on) conv_item(k, i, 0, prc);
+          else if (dout) append_tiles(task_tiles[k], VPZ_TILE_ZERO, dst_offsets[i], count[i], 0, count[i], files[t.file]->master.channels());
           continue;
         }
         d->current_position = 0;
@@ -1580,7 +1920,12 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
         }
         d->seg_sink = nullptr;
         if (got) got[i] = src ? src : have;
-        if (dout) {   // the segments (samples [0, have)), then zeros up to count
+        if (conv_on) {   // the window's segments into the scratch, then K6
+          const uint64_t item = (uint64_t)(dst_offsets[i] - g.base);
+          for (size_t sg = mark; sg < segs.size(); sg++)
+            append_tiles(task_xtiles[k], segs[sg].src, xoff[i], count[i], (segs[sg].dst - item) / C, segs[sg].n / C, C);
+          conv_item(k, i, src ? 0 : have, src);
+        } else if (dout) {   // the segments (samples [0, have)), then zeros up to count
           const uint64_t item = (uint64_t)(dst_offsets[i] - g.base);
           for (size_t sg = mark; sg < segs.size(); sg++)
             append_tiles(task_tiles[k], segs[sg].src, dst_offsets[i], count[i], (segs[sg].dst - item) / C, segs[sg].n / C, C);
@@ -1603,27 +1948,47 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
       }
       xb.h_segs[slot].n = n_segs;
     }
+    size_t n_dst_tiles = 0;   // K5 tiles into dst; the scratch's (task_xtiles) follow them
     if (dout) {
       size_t n_tiles = 0;
-      for (const auto& v : task_tiles) n_tiles += v.size();
+      for (const auto& v : task_tiles) n_dst_tiles += v.size();
+      n_tiles = n_dst_tiles;
+      for (const auto& v : task_xtiles) n_tiles += v.size();
       HostBuf<VpzPlaceTile>& ht = ctx->place->h_tiles[slot];
       if (!ht.reserve(n_tiles)) {
         rc = VPZ_E_NOMEM;
         break;
       }
       size_t at = 0;
-      for (const auto& v : task_tiles) {
-        if (!v.empty()) memcpy(ht.p + at, v.data(), v.size() * sizeof(VpzPlaceTile));
-        at += v.size();
-      }
+      for (const auto* vv : {&task_tiles, &task_xtiles})
+        for (const auto& v : *vv) {
+          if (!v.empty()) memcpy(ht.p + at, v.data(), v.size() * sizeof(VpzPlaceTile));
+          at += v.size();
+        }
       ht.n = n_tiles;
+      if (cv) {
+        size_t n_ct = 0;
+        for (const auto& v : task_ctiles) n_ct += v.size();
+        HostBuf<VpzConvTile>& hc = ctx->place->h_ctiles[slot];
+        if (!hc.reserve(n_ct)) {
+          rc = VPZ_E_NOMEM;
+          break;
+        }
+        at = 0;
+        for (const auto& v : task_ctiles) {
+          if (!v.empty()) memcpy(hc.p + at, v.data(), v.size() * sizeof(VpzConvTile));
+          at += v.size();
+        }
+        hc.n = n_ct;
+      }
     }
     tt1 = now(); t_deliver += tt1 - tt0; tt0 = tt1;
     if (dout) {
       // H2D + K1a + K1b + K3 (unclipped) + K5: the segments and zeros straight into the caller's device buffer
-      if (g.floats > 0) {
+      if (g.floats > 0 || (cv && ctx->place->h_ctiles[slot].n)) {
         if (b->total_floats && (rc = batch_decode(b, 0))) break;
-        if ((rc = place_tiles(ctx, slot, b, *dout, clip))) break;
+        if ((rc = place_tiles(ctx, slot, b, *dout, clip, n_dst_tiles))) break;
+        if (cv && (rc = convert_tiles(ctx, slot, ctx->place->d_scratch[slot].p, *dout))) break;
       }
       dev::event_record(xb.done[slot], ctx->stream);
       used[slot] = true;
@@ -1704,6 +2069,26 @@ int64_t vpz_decode_excerpts_device(vpz_ctx* ctx, uint32_t n_files, const uint8_t
                                                          static_cast<float*>(dst_dev), dst_elems, dst_offsets, got, &o));
 }
 
+int64_t vpz_decode_excerpts_device_conv(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
+                                        uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
+                                        int clip, const vpz_out_conv* conv, void* dst_dev, size_t dst_elems,
+                                        int64_t* dst_offsets, int32_t* got, void* stream) {
+  if (!ctx || !datas || !lens || (n && (!file_of || !start || !count))) return VPZ_E_ARGUMENT;
+  VPZ_USE(ctx);
+  int rc = conv_check(ctx, conv);
+  if (rc) return rc;
+  DevOut o;
+  o.p = dst_dev;
+  o.format = conv->format;
+  o.stream = stream;
+  o.conv = conv;
+  dev::Event* ev = nullptr;
+  rc = device_output_begin(ctx, o, &ev);
+  if (rc) return device_output_end(ctx, ev, rc);
+  return device_output_end(ctx, ev, decode_excerpts_impl(ctx, n_files, datas, lens, n, file_of, start, count, clip,
+                                                         static_cast<float*>(dst_dev), dst_elems, dst_offsets, got, &o));
+}
+
 // Debug / tests: the page-end granule index of one container image (first logical stream), built on the device
 // (K0 + K0g; VPZ_E_UNSUPPORTED when the file does not qualify) or by the host's packet walk.  Returns the number
 // of pages, writes min(pages, cap) entries.
@@ -1734,7 +2119,8 @@ int64_t vpz_debug_page_end_granules(vpz_ctx* ctx, const uint8_t* data, size_t le
 }  // extern "C"
 
 #ifdef VPZ_EMU
-// The emulated CPU test build (tests/emu, never linked into libvpz.so) takes the K5 launcher and the caller-memory
-// hooks of the device-output calls above from here.
+// The emulated CPU test build (tests/emu, never linked into libvpz.so) takes the K5 and K6 launchers and the
+// caller-memory hooks of the device-output calls above from here.
 #include "../../tests/emu/dev_emu_place.h"
+#include "../../tests/emu/dev_emu_convert.h"
 #endif

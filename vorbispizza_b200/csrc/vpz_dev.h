@@ -252,3 +252,29 @@ struct VpzPlaceTile {
   uint32_t n;               // samples
   uint32_t ch;              // channels
 };
+
+// ---- K6: rate and channel conversion into the caller's device buffer (k6_convert.cuh) ------------------------
+// Output j of an item at source rate fi and output rate fo (fi / fo = o / n in lowest terms) reads the 2 width + 2
+// source frames from floor(j o / n) - width on, weighted by phase j mod n of the rate pair's coefficient table.
+enum { VPZ_MIX_KEEP = 0, VPZ_MIX_MEAN = 1, VPZ_MIX_DUP = 2 };
+#define K6_SMEM_BUDGET 32768           // bytes of staged source a tile aims for (several CTAs per SM)
+#define K6_MAX_OUTS 4096               // output samples per tile at most
+#define K6_MAX_TAB_FLOATS (1u << 22)   // coefficient table of one rate pair at most
+struct VpzConvTile {
+  uint64_t src;             // float offset of the item's source frame 0 in the source buffer (interleaved fp32)
+  int64_t s_first;          // first staged frame, relative to the item's frame 0 (frames outside [0, src_len): zeros)
+  uint64_t base;            // element offset of the item in the destination
+  uint64_t len;             // output samples per channel of the item (channel stride of the planar layout)
+  uint64_t first;           // first output sample of the tile in the item
+  const float* taps;        // coefficient table, [2 width + 2][n] (tap-major); NULL: equal rates, no filter
+  uint32_t src_len;         // source frames of the item
+  uint32_t span;            // frames staged
+  uint32_t n;               // output samples of the tile
+  uint32_t valid;           // of them computed from the source; the rest are zero (an excerpt's got)
+  uint32_t ro, rn;          // o, n: fi / fo in lowest terms
+  uint32_t width;
+  uint32_t p0, r0;          // first output j0 of the tile: j0 mod n, (j0 * o) mod n
+  uint8_t ch_src, ch_out;   // channels of the source and of the output
+  uint8_t mix;              // VPZ_MIX_*
+  uint8_t pad[5];
+};
