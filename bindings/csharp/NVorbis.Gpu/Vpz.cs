@@ -147,6 +147,12 @@ namespace NVorbis.Gpu
         // the same with every item converted to conv->SampleRate / conv->Channels (0: keep) on the GPU (K6)
         [LibraryImport(Lib)] internal static partial long vpz_decode_files_device_conv(IntPtr ctx, uint n, byte** datas, nuint* lens, int clip, VpzOutConv* conv, IntPtr dstDev, nuint dstElems, long* sampleCounts, long* dstOffsets, IntPtr stream);
         [LibraryImport(Lib)] internal static partial long vpz_decode_excerpts_device_conv(IntPtr ctx, uint nFiles, byte** datas, nuint* lens, uint n, uint* fileOf, long* start, int* count, int clip, VpzOutConv* conv, IntPtr dstDev, nuint dstElems, long* dstOffsets, int* got, IntPtr stream);
+        // corpus: images opened once (scan, headers, setups, seek index, lengths; images resident on the GPU), excerpts many times
+        [LibraryImport(Lib)] internal static partial int vpz_corpus_open(IntPtr ctx, uint n, byte** datas, nuint* lens, int copy, out IntPtr corpus);
+        [LibraryImport(Lib)] internal static partial void vpz_corpus_close(IntPtr corpus);
+        [LibraryImport(Lib)] internal static partial long vpz_corpus_info(IntPtr corpus, int* channels, int* sampleRate, long* samples);
+        [LibraryImport(Lib)] internal static partial ulong vpz_corpus_device_bytes(IntPtr corpus);
+        [LibraryImport(Lib)] internal static partial long vpz_corpus_excerpts_device(IntPtr corpus, uint n, uint* fileOf, long* start, int* count, int clip, VpzOutConv* conv, IntPtr dstDev, nuint dstElems, long* dstOffsets, int* got, IntPtr stream);
         [LibraryImport(Lib)] internal static partial long vpz_debug_page_end_granules(IntPtr ctx, byte* data, nuint len, int onDevice, long* dst, nuint cap);
     }
 }

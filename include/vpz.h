@@ -381,6 +381,35 @@ int64_t vpz_decode_excerpts_device_conv(vpz_ctx* ctx, uint32_t n_files, const ui
                                         int clip, const vpz_out_conv* conv, void* dst_dev, size_t dst_elems,
                                         int64_t* dst_offsets, int32_t* got, void* stream);
 
+/* ---- corpus: open a set of container images once, cut excerpt batches from it many times --------------------- */
+typedef struct vpz_corpus vpz_corpus;
+/* Opens n container images as one corpus of the context.  Does once what every excerpt call does per call: the page
+ * scan (on the device, or on the host with "gpu_scan" 0), the headers and setup tables (the corpus holds its
+ * references until close), the seek index (built on the device for clean single-stream files, by the host's packet
+ * walk for the rest) and each file's total samples.  The images are scanned in slices of at most "bulk_group_mib"
+ * (the pinned staging never holds the whole corpus); the 4 GiB limit per image stays.  A file the plain excerpt call
+ * rejects fails the open with the same code and last-error text, and *out stays NULL.
+ *   copy != 0: the library keeps its own copy of the images.  copy == 0: the caller's bytes must stay valid and
+ *   unchanged until vpz_corpus_close (vpz_reader_open_memory's rules).
+ * A corpus belongs to its context: every call on it is a call on that context (one thread at a time), and it must be
+ * closed before the context is destroyed.  The settings in effect at open ("gpu_scan", "bulk_group_mib") apply. */
+int vpz_corpus_open(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int copy,
+                    vpz_corpus** out);
+void vpz_corpus_close(vpz_corpus* c);
+/* Per file: channels, sample rate, TotalSamples of a fresh reader on its first logical stream (any pointer may be
+ * NULL).  Returns the number of files. */
+int64_t vpz_corpus_info(const vpz_corpus* c, int32_t* channels, int32_t* sample_rate, int64_t* samples);
+/* Bytes of device memory the corpus holds (its images, 16-byte aligned with 16 zero bytes behind each); 0 for NULL. */
+uint64_t vpz_corpus_device_bytes(const vpz_corpus* c);
+/* vpz_decode_excerpts_device_conv on the corpus's files: same arguments after (n_files, datas, lens), same results.
+ * Given the same images the buffer, got, dst_offsets, the size query (dst_dev == NULL), the error codes and
+ * ClipSamples are bitwise those of vpz_decode_excerpts_device_conv; with conv = {format, 0, 0} that is also the plain
+ * vpz_decode_excerpts_device(format).  A call costs the planning and decoding of its excerpts: nothing of a file is
+ * scanned, parsed or indexed again.  NULL c: VPZ_E_ARGUMENT. */
+int64_t vpz_corpus_excerpts_device(vpz_corpus* c, uint32_t n, const uint32_t* file_of, const int64_t* start,
+                                   const int32_t* count, int clip, const vpz_out_conv* conv, void* dst_dev,
+                                   size_t dst_elems, int64_t* dst_offsets, int32_t* got, void* stream);
+
 /* Debug / tests: the page-end granule index SeekTo searches in (PacketProvider.FillPageEndGranuleCache,
  * Ogg/PacketProvider.cs:203-307) of one container image's first logical stream: entry p = granules up to and
  * including page p.  on_device 1: built by the GPU (page scan + one warp per file over its pages), VPZ_E_UNSUPPORTED

@@ -10,6 +10,7 @@ from ._native import VpzError, load  # noqa: F401
 from .api import (  # noqa: F401
     Batch,
     Context,
+    Corpus,
     InvalidDataError,
     PreRollPacketError,
     SeekOutOfRangeError,
@@ -22,6 +23,6 @@ from .api import (  # noqa: F401
     scan_pages,
 )
 
-__all__ = ["Batch", "Context", "SynthBatch", "VorbisReader", "decode_files", "decode_excerpts", "decode_files_device",
+__all__ = ["Batch", "Context", "Corpus", "SynthBatch", "VorbisReader", "decode_files", "decode_excerpts", "decode_files_device",
            "decode_excerpts_device", "scan_pages", "VpzError", "InvalidDataError",
            "SeekOutOfRangeError", "PreRollPacketError", "load"]

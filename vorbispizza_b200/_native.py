@@ -134,6 +134,12 @@ _SIGS = {
                                                  _P, _P, _P]),
     "vpz_decode_excerpts_device_conv": (C.c_int64, [_P, C.c_uint32, _P, _P, C.c_uint32, _P, _P, _P, C.c_int,
                                                     C.POINTER(OutConv), _P, C.c_size_t, _P, _P, _P]),
+    "vpz_corpus_open": (C.c_int, [_P, C.c_uint32, _P, _P, C.c_int, C.POINTER(_P)]),
+    "vpz_corpus_close": (None, [_P]),
+    "vpz_corpus_info": (C.c_int64, [_P, _P, _P, _P]),
+    "vpz_corpus_device_bytes": (C.c_uint64, [_P]),
+    "vpz_corpus_excerpts_device": (C.c_int64, [_P, C.c_uint32, _P, _P, _P, C.c_int, C.POINTER(OutConv), _P, C.c_size_t,
+                                               _P, _P, _P]),
     "vpz_debug_page_end_granules":(C.c_int64, [_P, _P, C.c_size_t, C.c_int, _P, C.c_size_t]),
     "vpz_scan_pages": (C.c_int64, [_P, C.c_uint32, _P, _P, _P, C.c_size_t, _P, _P, _P, _P]),
 }

@@ -6,6 +6,7 @@ IsEndOfStream, TotalSamples, SamplePosition ...), spelled the Python way.  Error
 reference's exception types the way INTEGRATION.md lists them.
 """
 import ctypes as C
+import weakref
 
 import numpy as np
 
@@ -51,6 +52,7 @@ class Context:
         if rc:
             raise N.VpzError(rc, self.lib.vpz_strerror(rc).decode())
         self._h = h
+        self._corpora = weakref.WeakSet()   # open Corpus objects: closed before the context
 
     def check(self, rc):
         if rc is not None and rc < 0:
@@ -63,6 +65,8 @@ class Context:
 
     def close(self):
         if self._h:
+            for c in list(self._corpora):   # a corpus must be closed before its context
+                c.close()
             self.lib.vpz_ctx_destroy(self._h)
             self._h = None
 
@@ -607,6 +611,86 @@ def decode_excerpts_device(ctx, files, file_of, start, count, clip=True, dtype="
     buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
     total = ctx.check(fn(*args, ptr, elems, offsets.ctypes.data, got.ctypes.data, handle))
     return buf[:total], offsets, got
+
+
+class Corpus:
+    """vpz_corpus: container images opened once (page scan, headers, setup tables, seek index, total samples) and
+    cut into excerpt batches many times, each call costing only its excerpts' planning and decoding.
+
+    files: list of bytes / uint8 arrays.  copy=False keeps references to the caller's buffers, which must not change
+    while the corpus is open; copy=True makes the library keep its own copy.  close() (or dropping the corpus) frees
+    its device memory; closing the context closes its open corpora first.
+    .channels, .sample_rates and .samples (TotalSamples) are per-file numpy arrays, for drawing crops uniformly."""
+
+    def __init__(self, ctx, files, copy=False):
+        self.ctx = ctx
+        self._h = None
+        keep = [_u8(f) for f in files]
+        n = len(keep)
+        ptrs = (C.c_void_p * max(n, 1))(*[k[1] for k in keep])
+        lens = (C.c_size_t * max(n, 1))(*[k[2] for k in keep])
+        h = C.c_void_p()
+        ctx.check(ctx.lib.vpz_corpus_open(ctx._h, n, ptrs, lens, int(bool(copy)), C.byref(h)))
+        self._h = h
+        self._keep = None if copy else keep
+        ctx._corpora.add(self)
+        self.channels = np.zeros(n, np.int32)
+        self.sample_rates = np.zeros(n, np.int32)
+        self.samples = np.zeros(n, np.int64)
+        ctx.check(ctx.lib.vpz_corpus_info(h, self.channels.ctypes.data, self.sample_rates.ctypes.data,
+                                          self.samples.ctypes.data))
+
+    def __len__(self):
+        return self.samples.size
+
+    @property
+    def device_bytes(self):
+        """Bytes of device memory the corpus holds (its images)."""
+        return int(self.ctx.lib.vpz_corpus_device_bytes(self._h)) if self._h else 0
+
+    def close(self):
+        """Frees the device images and the setup references; Context.close() closes its open corpora first."""
+        if self._h:
+            self.ctx.lib.vpz_corpus_close(self._h)
+            self._h = None
+            self._keep = None
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def __del__(self):   # a dropped corpus gives its device memory back (its context is still open: it closes corpora first)
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def excerpts(self, file_of, start, count, clip=True, dtype="float32", planar=True, out=None, stream=None,
+                 sample_rate=None, channels=None):
+        """vpz_corpus_excerpts_device: decode_excerpts_device on the corpus's files, same arguments after `files`
+        and bitwise the same (buf, offsets, got)."""
+        if not self._h:
+            raise ValueError("corpus is closed")
+        ctx = self.ctx
+        file_of = np.ascontiguousarray(file_of, dtype=np.uint32)
+        start = np.ascontiguousarray(start, dtype=np.int64)
+        count = np.ascontiguousarray(count, dtype=np.int32)
+        n = file_of.size
+        offsets = np.zeros(n, np.int64)
+        got = np.zeros(n, np.int32)
+        fmt = _format(dtype, planar)
+        conv = N.OutConv(fmt, int(sample_rate or 0), int(channels or 0))
+        args = (self._h, n, file_of.ctypes.data, start.ctypes.data, count.ctypes.data, int(bool(clip)), C.byref(conv))
+        total = None
+        if out is None:
+            total = ctx.check(ctx.lib.vpz_corpus_excerpts_device(*args, None, 0, offsets.ctypes.data, got.ctypes.data,
+                                                                 None))
+        buf, ptr, elems, handle = _device_out(ctx, out, total, dtype, stream)
+        total = ctx.check(ctx.lib.vpz_corpus_excerpts_device(*args, ptr, elems, offsets.ctypes.data, got.ctypes.data,
+                                                             handle))
+        return buf[:total], offsets, got
 
 
 PAGE_DTYPE = np.dtype([("offset", "<u4"), ("body_len", "<u4"), ("granule", "<i8"), ("serial", "<u4"), ("sequence", "<u4"),

@@ -13,6 +13,7 @@
 #include "k4_deliver.cuh"
 #include "k5_place.cuh"
 #include "k6_convert.cuh"
+#include "k7_gather.cuh"
 
 // ---- kernels ---------------------------------------------------------------------------------
 __global__ void __launch_bounds__(K0_THREADS) vpz_k0_pages(K0Params P) {
@@ -31,6 +32,8 @@ __global__ void __launch_bounds__(K4_THREADS) vpz_k4_deliver(K4Params P) { k4_ct
 
 template <bool OUT16, bool PLANAR>
 __global__ void __launch_bounds__(K5_THREADS) vpz_k5_place(K5Params P) { k5_cta<OUT16, PLANAR>(P); }
+
+__global__ void __launch_bounds__(K7_THREADS) vpz_k7_gather(K7Params P) { k7_cta(P); }
 
 template <bool OUT16, bool PLANAR>
 __global__ void __launch_bounds__(K6_THREADS) vpz_k6_convert(K6Params P) {
@@ -330,6 +333,15 @@ int launch_k5(const K5Params& p, Stream* s, std::string& err) {
   }
   cudaError_t e = cudaGetLastError();
   return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k5_place", err);
+}
+
+int launch_k7(const K7Params& p, Stream* s, std::string& err) {
+  if (p.n_pieces == 0) return VPZ_OK;
+  const unsigned warps = K7_THREADS / 32;
+  unsigned grid = (unsigned)std::min<size_t>(((size_t)p.n_pieces + warps - 1) / warps, (size_t)8 * sm_count());
+  vpz_k7_gather<<<grid, K7_THREADS, 0, s->s>>>(p);
+  cudaError_t e = cudaGetLastError();
+  return e == cudaSuccess ? VPZ_OK : fail(e, "launch vpz_k7_gather", err);
 }
 
 int launch_k6(const K6Params& p, Stream* s, std::string& err) {

@@ -73,6 +73,9 @@ int launch_k5(const K5Params& p, Stream* s, std::string& err);
 // K6: rate / channel conversion of tiles into the caller's device buffer, one CTA per tile, p.smem_floats * 4 bytes of
 // dynamic shared memory (VPZ_E_UNSUPPORTED when that exceeds the device's limit)
 int launch_k6(const K6Params& p, Stream* s, std::string& err);
+// K7: packet bytes of a corpus call from the corpus's device images into the batch's packet-byte area, one warp per
+// packet
+int launch_k7(const K7Params& p, Stream* s, std::string& err);
 
 // Caller-owned device memory (the *_device bulk calls): 0 when p is device or managed memory of `device`,
 // VPZ_E_ARGUMENT (with the reason in err) for host, pinned or another device's memory

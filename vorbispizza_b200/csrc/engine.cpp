@@ -481,20 +481,24 @@ int batch_commit(vpz_batch* b, RunPlan* const* plans, size_t n, ThreadPool* pool
     return VPZ_E_ARGUMENT;
   }
   const size_t old_bytes = b->bytes.n;
-  if (!b->bytes.reserve(bytes) || !b->pkts_in.reserve(pkt) || !b->pkts_ola.reserve(pkt) || !b->items.reserve(item))
+  const bool gather = b->gather_images != nullptr;   // K7 writes the bytes: nothing to stage
+  if ((!gather && !b->bytes.reserve(bytes)) || !b->pkts_in.reserve(pkt) || !b->pkts_ola.reserve(pkt) ||
+      !b->items.reserve(item))
     return VPZ_E_NOMEM;
   b->sort_key.resize(pkt);
-  memset(b->bytes.p + old_bytes, 0, (size_t)base[0].bytes - old_bytes);
+  if (!gather) memset(b->bytes.p + old_bytes, 0, (size_t)base[0].bytes - old_bytes);
   auto fill = [&](size_t i) {
     const RunPlan& p = *plans[i];
     const Base& bs = base[i];
     const size_t nv = p.src.size();
-    uint8_t* dst = b->bytes.p + bs.bytes;
+    uint8_t* dst = gather ? nullptr : b->bytes.p + bs.bytes;
     for (size_t k = 0; k < nv; k++) {
       const uint32_t off = p.byte_off[k], len = p.src[k].len;
       const uint32_t next = k + 1 < nv ? p.byte_off[k + 1] : (uint32_t)p.staged_bytes;
-      if (len) memcpy(dst + off, p.src[k].p, len);
-      memset(dst + off + len, 0, next - off - len);
+      if (!gather) {
+        if (len) memcpy(dst + off, p.src[k].p, len);
+        memset(dst + off + len, 0, next - off - len);
+      }
       VpzPktIn in;
       in.byte_off = (uint32_t)(bs.bytes + off);
       in.byte_len = len;
@@ -511,6 +515,7 @@ int batch_commit(vpz_batch* b, RunPlan* const* plans, size_t n, ThreadPool* pool
       b->sort_key[bs.pkt + k] = (((uint32_t)bs.slot * 2u + ((ola.flags & VPZ_OLA_LONG) ? 0u : 1u)) << 13) |
                                 (4096u - std::min<uint32_t>(len >> 2, 4096u));
     }
+    if (gather) b->gather_fill(i, bs.bytes);
     // K3 work items: packets 1..nv-1 emit; each item re-runs its predecessor as carry seed
     size_t it_idx = bs.item;
     for (size_t k = 1; k < nv; k += chunk) {
@@ -527,7 +532,10 @@ int batch_commit(vpz_batch* b, RunPlan* const* plans, size_t n, ThreadPool* pool
     pool->parallel_for(n, fill);
   else
     for (size_t i = 0; i < n; i++) fill(i);
-  b->bytes.n = bytes;
+  if (gather)
+    b->gather_bytes = bytes;
+  else
+    b->bytes.n = bytes;
   b->pkts_in.n = b->pkts_ola.n = pkt;
   b->items.n = item;
   b->spec_floats = spec;
@@ -578,8 +586,20 @@ int batch_upload(vpz_batch* b) {
   const size_t np = b->pkts_ola.n;
   int rc;
   if (!b->synthetic) {
-    if (!b->d_bytes.reserve(b->bytes.n + 16, err) || !b->d_pkts_in.reserve(np * sizeof(VpzPktIn), err)) return VPZ_E_CUDA;
-    if ((rc = dev::h2d(b->d_bytes.p, b->bytes.p, b->bytes.n, st, err))) return rc;
+    if (!b->d_bytes.reserve((b->gather_images ? b->gather_bytes : b->bytes.n) + 16, err) || !b->d_pkts_in.reserve(np * sizeof(VpzPktIn), err)) return VPZ_E_CUDA;
+    if (b->gather_images) {   // corpus call: K7 gathers the packet bytes from the corpus's device images
+      if (!b->d_pieces.reserve(b->pieces.n * sizeof(VpzGatherPiece), err)) return VPZ_E_CUDA;
+      if ((rc = dev::h2d(b->d_pieces.p, b->pieces.p, b->pieces.n * sizeof(VpzGatherPiece), st, err))) return rc;
+      K7Params kp;
+      kp.images = b->gather_images;
+      kp.bytes = static_cast<uint8_t*>(b->d_bytes.p);
+      kp.pieces = static_cast<const VpzGatherPiece*>(b->d_pieces.p);
+      kp.n_pieces = (uint32_t)b->pieces.n;
+      if ((rc = dev::launch_k7(kp, st, err))) return rc;
+      ctx->kernel_launches++;
+    } else if ((rc = dev::h2d(b->d_bytes.p, b->bytes.p, b->bytes.n, st, err))) {
+      return rc;
+    }
     if ((rc = dev::h2d(b->d_pkts_in.p, b->pkts_in.p, np * sizeof(VpzPktIn), st, err))) return rc;
     if (!b->d_res.reserve(np * sizeof(VpzPktRes), err)) return VPZ_E_CUDA;
     if (!b->d_spec.reserve(b->spec_floats * 4, err)) return VPZ_E_CUDA;

@@ -76,6 +76,7 @@ struct ScanResult {                  // views into the context's scan buffers, v
   const VpzScanFile* files = nullptr;
   const VpzPageRec* pages = nullptr;
   const VpzScanOut* out = nullptr;
+  const uint8_t* images = nullptr;   // the staged images on the device: image i at files[i].data_off
 };
 }  // namespace vpz
 
@@ -247,6 +248,16 @@ struct vpz_batch {
   vpz::HostBuf<const void*> h_setups;
   vpz::HostBuf<uint32_t> h_clip;
   bool clip_fetched = false;
+  // corpus calls (vpz_corpus_excerpts_device): set before batch_commit on an empty batch, K7 writes the packet bytes
+  // from the corpus's device images.  batch_commit then lays the packets out but stages none of their bytes (their
+  // layout size goes to gather_bytes, `bytes` stays empty) and calls gather_fill(plan, byte base of its run) from
+  // the thread that fills that plan, which writes the plan's pieces (one per packet and page) into `pieces`;
+  // batch_upload uploads the pieces instead of the bytes and launches K7.
+  const uint8_t* gather_images = nullptr;
+  uint64_t gather_bytes = 0;
+  std::function<void(size_t, uint64_t)> gather_fill;
+  vpz::HostBuf<VpzGatherPiece> pieces;
+  vpz::DevBuf d_pieces;
   float ms_k1 = 0, ms_k1a = 0, ms_k1b = 0, ms_k3 = 0, ms_total = 0;
   int launches = 0;
   // debug plumbing (vpz_debug_decode_packet)

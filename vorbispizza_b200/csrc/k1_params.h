@@ -89,6 +89,13 @@ struct K6Params {
   int out16;                       // 1: int16 elements by K3's rule (k3_s16)
 };
 
+struct K7Params {
+  const uint8_t* images;           // the corpus's images: 16-byte aligned, zeros behind each
+  uint8_t* bytes;                  // the batch's packet-byte area (K1a's input)
+  const VpzGatherPiece* pieces;
+  uint32_t n_pieces;
+};
+
 struct K0gParams {
   const uint8_t* images;           // the staged images of the K0 scan
   const VpzGranFile* files;

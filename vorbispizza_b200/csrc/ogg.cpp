@@ -263,7 +263,7 @@ int LogicalStream::load_pages_upto(int64_t idx) {
       has_all_pages = true;  // SetEndOfStreams at the physical end
       break;
     }
-    OggPage& p = pages[(size_t)pages_loaded];
+    const OggPage& p = pages[(size_t)pages_loaded];
     if (p.granule != -1) {
       if (first_data_page < 0 && p.granule > 0) {
         first_data_page = pages_loaded;
@@ -277,7 +277,7 @@ int LogicalStream::load_pages_upto(int64_t idx) {
     if (p.flags & 4) has_all_pages = true;
     if (pages_loaded > 0) {
       uint32_t last = pages[(size_t)pages_loaded - 1].seq;
-      if (last != 0 && last + 1 != p.seq) p.is_resync = true;
+      if (last != 0 && last + 1 != p.seq) pages.mut((size_t)pages_loaded).is_resync = true;
     }
     container_bits += 8 * (27 + p.nseg);
     pages_loaded++;
@@ -347,6 +347,8 @@ void LogicalStream::create_packet(int64_t* pg, int* pk, bool advance, int64_t gr
       if (!(np->flags & 1) || is_resync) break;
       if (is_continued && packet_count > 1) is_continued = false;
       page_packet_slice(np, 0, &d, &n);
+      if (out->spans.empty()) out->spans.push_back(OggSpan{out->ptr, out->len});
+      out->spans.push_back(OggSpan{d, (uint32_t)n});
       if (out->owned.empty() && out->len) out->owned.assign(out->ptr, out->ptr + out->len);
       out->owned.insert(out->owned.end(), d, d + n);
       out->len = (uint32_t)out->owned.size();

@@ -7,6 +7,7 @@
 #include <stdint.h>
 
 #include <functional>
+#include <memory>
 #include <vector>
 
 #include "vpz_dev.h"
@@ -27,12 +28,18 @@ struct OggPage {
   bool is_continued = false;
 };
 
+struct OggSpan {   // bytes of the container image
+  const uint8_t* p = nullptr;
+  uint32_t len = 0;
+};
+
 struct OggPacket {
   // A packet that lies inside one page is a VIEW into the container image (no copy); only packets
   // continued across pages are assembled into `owned`.
   const uint8_t* ptr = nullptr;
   uint32_t len = 0;
   std::vector<uint8_t> owned;
+  std::vector<OggSpan> spans;   // a packet continued across pages: its bytes on each page, in order (views)
   const uint8_t* data() const { return ptr; }
   size_t size() const { return len; }
   bool valid = false;
@@ -44,11 +51,34 @@ struct OggPacket {
 
 uint32_t ogg_crc(const uint8_t* data, size_t len, uint32_t crc = 0);
 
+// A vector that copies of its owner share until one of them writes (copy on write): a copy of a LogicalStream is a
+// new packet cursor over the same page list and page-end index, whatever the length of the file.  Writers copy first,
+// so a shared vector is never written; concurrent copies of one unchanged master are safe.
+template <class T>
+class SharedVec {
+ public:
+  size_t size() const { return v_->size(); }
+  bool empty() const { return v_->empty(); }
+  const T& operator[](size_t i) const { return (*v_)[i]; }
+  T& mut(size_t i) { return own()[i]; }
+  void push_back(const T& x) { own().push_back(x); }
+  template <class It>
+  void assign(It first, It last) { own().assign(first, last); }
+  operator const std::vector<T>&() const { return *v_; }
+
+ private:
+  std::shared_ptr<std::vector<T>> v_ = std::make_shared<std::vector<T>>();
+  std::vector<T>& own() {
+    if (v_.use_count() > 1) v_ = std::make_shared<std::vector<T>>(*v_);
+    return *v_;
+  }
+};
+
 // One logical bitstream (one serial number, BOS..EOS) = StreamPageReader + PacketProvider.
 class LogicalStream {
  public:
   uint32_t serial = 0;
-  std::vector<OggPage> pages;       // every page the physical reader would hand to this stream
+  SharedVec<OggPage> pages;         // every page the physical reader would hand to this stream
   // lazily "read" prefix: HasAllPages / IsEndOfStream in the reference depend on how far the
   // reader has got (StreamPageReader.cs:82-85,249,442-446)
   int64_t pages_loaded = 0;
@@ -59,7 +89,7 @@ class LogicalStream {
   // packet cursor (PacketProvider._pageIndex/_packetIndex)
   int64_t page_index = 0;
   int packet_index = 0;
-  std::vector<int64_t> page_end_granules;
+  SharedVec<int64_t> page_end_granules;
   // IPacketGranuleCountProvider.GetPacketGranuleCount (set by the decoder)
   std::function<int(const OggPacket&)> granule_count;
 

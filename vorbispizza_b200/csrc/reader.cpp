@@ -28,6 +28,7 @@
 #include <new>
 #include <numeric>
 #include <thread>
+#include <unordered_map>
 
 #include "../../include/vpz.h"
 #include "bitreader.h"
@@ -64,6 +65,7 @@ struct Window {
   std::vector<int32_t> trims;
   std::vector<int> entry_of;      // submitted packet -> entry index (-1: carried-over seed packet)
   std::vector<std::vector<uint8_t>> arena;  // packets assembled across pages (moving an inner vector keeps its buffer: the views stay valid)
+  std::vector<std::vector<OggSpan>> arena_spans;   // per arena packet: its bytes on each page of the image (K7's pieces)
   // drain of the last decoded packet's raw right half (see resolve_drain)
   bool drain = false, drain_extra_run = false;
   int drain_tail = 0, drain_entry = -1;
@@ -75,6 +77,7 @@ struct Window {
   void add_packet(OggPacket* pk, int32_t trim, int entry) {
     if (!pk->owned.empty()) {
       arena.push_back(std::move(pk->owned));
+      arena_spans.push_back(std::move(pk->spans));
       src.push_back(PktSrc{arena.back().data(), (uint32_t)arena.back().size()});
     } else {
       src.push_back(PktSrc{pk->ptr, pk->len});
@@ -1491,6 +1494,7 @@ struct ExcerptJob {
   int64_t pos = 0;             // granule position the provider reported for the target packet
   int status = 0;              // error of the provider side of SeekTo
   int run = -1, drain_run = -1;
+  size_t pieces[2] = {0, 0};   // corpus call: K7 pieces of the window's plan / drain plan, SIZE_MAX: not in the image
 };
 struct ExcerptTask {           // consecutive excerpts of one file, handled by one worker with its own cursor
   uint32_t file = 0;
@@ -1526,8 +1530,10 @@ static bool clean_single_stream(const ExcerptFile& f, const VpzPageRec* r, uint3
 
 // Opens the files of a random-access batch: page scan (K0, or the host with "gpu_scan" 0), headers and setup
 // tables, and the page-end granule index SeekTo searches in (K0g for clean files; files_on_device counts them).
+// scan: the device scan's result (its staged images stay on the device until the next scan), when there was one.
 static int open_excerpt_files(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
-                              std::vector<std::unique_ptr<ExcerptFile>>& files, uint32_t* files_on_device) {
+                              std::vector<std::unique_ptr<ExcerptFile>>& files, uint32_t* files_on_device,
+                              ScanResult* scan = nullptr) {
   ThreadPool* pool = ctx->pool;
   ScanResult sr;
   const bool dev_scan = ctx->gpu_scan != 0 && n_files > 0;
@@ -1601,16 +1607,88 @@ static int open_excerpt_files(vpz_ctx* ctx, uint32_t n_files, const uint8_t* con
     if (err) return err;
   }
   if (files_on_device) *files_on_device = on_device;
+  if (scan && dev_scan) *scan = sr;
   return VPZ_OK;
 }
 
 }  // extern "C"
 
-// dout: the caller's device buffer instead of dst (dst is its address): K5 places the segments and zero-fills
+// ---- corpus: the files of the excerpt calls opened once ----------------------------------------------------------
+// vpz_corpus_open runs open_excerpt_files (page scan, headers, setup tables, seek index, total samples) once and keeps
+// the images in device memory; every vpz_corpus_excerpts_device call then starts at the excerpt planning with the
+// same opened files the plain call would have built, and K7 gathers its packet bytes from the device images.  The
+// calls only read the files: each planning task copies a file's packet cursor, the masters stay as open left them, so
+// one call leaves nothing behind for the next.
+struct vpz_corpus {
+  vpz_ctx* ctx = nullptr;
+  std::vector<std::vector<uint8_t>> copies;   // copy != 0: the library's own images
+  std::vector<std::unique_ptr<ExcerptFile>> files;
+  std::vector<int64_t> samples;               // TotalSamples per file
+  uint8_t* d_img = nullptr;                   // the images on the device: 16-byte aligned, >= 16 zero bytes behind each
+  uint64_t d_bytes = 0;
+  std::vector<uint64_t> dev_off;              // per file: offset of its image in d_img
+  ~vpz_corpus() {
+    if (ctx) VPZ_USE(ctx);
+    files.clear();                            // gives the setup tables back to the context
+    dev::free(d_img);
+  }
+};
+
+// K7's pieces of one packet of a window: a view of the file's image is one piece, a packet assembled across pages one
+// per page (its spans); n_pieces returns 0 when the packet is not in the image (the group then stages it on the host).
+static const std::vector<OggSpan>* packet_spans(const Window& w, const uint8_t* p) {
+  for (size_t a = 0; a < w.arena.size(); a++)
+    if (w.arena[a].data() == p) return &w.arena_spans[a];
+  return nullptr;
+}
+static bool in_image(const OggContainer& c, const uint8_t* p, uint32_t len) {
+  return len == 0 || (p >= c.data && p + len <= c.data + c.len);
+}
+static size_t n_pieces(const OggContainer& c, const Window& w, const PktSrc& ps) {
+  if (in_image(c, ps.p, ps.len)) return 1;
+  const std::vector<OggSpan>* sp = packet_spans(w, ps.p);
+  if (!sp || sp->empty()) return 0;
+  for (const OggSpan& x : *sp)
+    if (!in_image(c, x.p, x.len)) return 0;
+  return sp->size();
+}
+static size_t plan_pieces(const OggContainer& c, const Window& w, const RunPlan& plan) {
+  size_t n = 0;
+  for (const PktSrc& ps : plan.src) {
+    const size_t k = n_pieces(c, w, ps);
+    if (!k) return SIZE_MAX;
+    n += k;
+  }
+  return n;
+}
+// writes the pieces of `plan` (committed at byte `base` of the batch) from `pc` on; returns the packets over pages
+static size_t put_pieces(const OggContainer& c, uint64_t img, const Window& w, const RunPlan& plan, uint64_t base,
+                         VpzGatherPiece* pc) {
+  size_t multi = 0;
+  for (size_t q = 0; q < plan.src.size(); q++) {
+    const PktSrc& ps = plan.src[q];
+    uint32_t off = (uint32_t)(base + plan.byte_off[q]);
+    if (in_image(c, ps.p, ps.len)) {
+      *pc++ = VpzGatherPiece{ps.len ? img + (uint64_t)(ps.p - c.data) : img, off, ps.len};
+      continue;
+    }
+    const std::vector<OggSpan>& sp = *packet_spans(w, ps.p);
+    for (size_t i = 0; i < sp.size(); i++) {
+      *pc++ = VpzGatherPiece{sp[i].len ? img + (uint64_t)(sp[i].p - c.data) : img, off,
+                             sp[i].len | (i + 1 < sp.size() ? VPZ_PIECE_MORE : 0u)};
+      off += sp[i].len;
+    }
+    multi++;
+  }
+  return multi;
+}
+
+// dout: the caller's device buffer instead of dst (dst is its address): K5 places the segments and zero-fills.
+// corpus: its files (vpz_corpus_open) instead of datas / lens, and K7 instead of the packet bytes' staging.
 static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_t* const* datas, const size_t* lens,
                                     uint32_t n, const uint32_t* file_of, const int64_t* start, const int32_t* count,
                                     int clip, float* dst, size_t dst_floats, int64_t* dst_offsets, int32_t* got,
-                                    const DevOut* dout) {
+                                    const DevOut* dout, vpz_corpus* corpus = nullptr) {
   if (!ctx->pool) {
     unsigned t = ctx->host_threads > 0 ? (unsigned)ctx->host_threads
                                        : std::max(1u, std::min(std::thread::hardware_concurrency(), 32u));
@@ -1622,9 +1700,11 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
   auto now = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   double t_files = 0, t_tasks = 0, t_plan = 0, t_commit = 0, t_launch = 0, t_wait = 0, t_deliver = 0, tt0 = now(), tt1;
   // ---- files: page scan, headers, setup tables, seek index (once per file) ---------------------------
-  std::vector<std::unique_ptr<ExcerptFile>> files(n_files);
-  {
-    int rc = open_excerpt_files(ctx, n_files, datas, lens, files, nullptr);
+  std::vector<std::unique_ptr<ExcerptFile>> own_files;
+  std::vector<std::unique_ptr<ExcerptFile>>& files = corpus ? corpus->files : own_files;
+  if (!corpus) {
+    own_files.resize(n_files);
+    int rc = open_excerpt_files(ctx, n_files, datas, lens, own_files, nullptr);
     if (rc) return rc;
   }
   tt1 = now(); t_files = tt1 - tt0; tt0 = tt1;
@@ -1778,6 +1858,11 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
         std::string err;
         int rc = plan_submit(d, j.win.get(), &err);
         if (rc) j.status = rc;
+        if (!rc && corpus) {   // K7's pieces of the window (SIZE_MAX: a packet outside the image)
+          const OggContainer& c = files[t.file]->cont;
+          if (j.win->has_plan) j.pieces[0] = plan_pieces(c, *j.win, j.win->plan);
+          if (j.win->has_drain_plan) j.pieces[1] = plan_pieces(c, *j.win, j.win->drain_plan);
+        }
       }
     });
   };
@@ -1798,6 +1883,8 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
   std::vector<std::vector<VpzPlaceTile>> task_tiles, task_xtiles;   // K5 into dst / into the scratch (_conv)
   std::vector<std::vector<VpzConvTile>> task_ctiles;                 // K6 (_conv)
   std::vector<uint64_t> xoff(cv ? n : 0);                             // float offset of a converted excerpt's window in the scratch
+  uint64_t gathered_bytes = 0, gathered_pieces = 0;                   // K7 (corpus call): staged bytes written, pieces,
+  uint64_t gathered_multi = 0, gathered_groups = 0;                   // packets over pages, groups it gathered
   for (size_t gi = 0; gi < groups.size() && !rc; gi++) {
     const Group& g = groups[gi];
     const int slot = (int)(gi & 1);
@@ -1834,9 +1921,40 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
           owner.push_back({&j, 1});
         }
       }
+    // corpus call: K7 gathers the packet bytes from the corpus's device images instead of the host staging them,
+    // when every packet of the group lies in its file's image (a view, or assembled from views of several pages);
+    // batch_commit's fill threads write each plan's pieces
+    bool gather = corpus && corpus->d_img && b->bytes.n == 0;
+    std::vector<size_t> piece_at(gather ? plans.size() + 1 : 0);   // per plan: its first piece
+    for (size_t k = 0; k < plans.size() && gather; k++) {
+      const size_t np = owner[k].first->pieces[owner[k].second];
+      gather = np != SIZE_MAX;
+      piece_at[k + 1] = piece_at[k] + (gather ? np : 0);
+    }
+    std::atomic<size_t> multi{0};
+    if (gather) {
+      if (!b->pieces.reserve(piece_at.back())) {
+        rc = VPZ_E_NOMEM;
+        break;
+      }
+      b->pieces.n = piece_at.back();
+      b->gather_images = corpus->d_img;
+      b->gather_fill = [&](size_t k, uint64_t base) {
+        const ExcerptJob& j = *owner[k].first;
+        const uint32_t f = file_of[j.index];
+        multi += put_pieces(files[f]->cont, corpus->dev_off[f], *j.win, *plans[k], base, b->pieces.p + piece_at[k]);
+      };
+    }
     int first = 0;
     if ((rc = batch_commit(b, plans.data(), plans.size(), pool, &first))) break;
     for (size_t k = 0; k < owner.size(); k++) (owner[k].second ? owner[k].first->drain_run : owner[k].first->run) = first + (int)k;
+    if (gather) {
+      b->gather_fill = nullptr;
+      gathered_bytes += b->gather_bytes;
+      gathered_pieces += piece_at.back();
+      gathered_multi += multi;
+      gathered_groups++;
+    }
     tt1 = now(); t_commit += tt1 - tt0; tt0 = tt1;
     // consumer side, samples untouched: SeekTo's two packets, then Read until `count` samples or the end
     task_segs.assign(g.t1 - g.t0, std::vector<VpzCopySeg>());
@@ -2033,9 +2151,15 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
   int r2 = dev::stream_sync(ctx->stream, ctx->last_error);
   if (!rc) rc = r2;
   t_wait += now() - tt0;
-  if (trace)
-    fprintf(stderr, "vpz_decode_excerpts%s: %u excerpts, %zu tasks, %zu groups: files %.1f tasks %.1f plan %.1f commit %.1f replay %.1f launch %.1f wait %.1f ms\n",
-            dout ? "_device" : "", n, tasks.size(), groups.size(), t_files, t_tasks, t_plan, t_commit, t_deliver, t_launch, t_wait);
+  if (trace) {
+    fprintf(stderr, "vpz_decode_excerpts%s: %u excerpts, %zu tasks, %zu groups: files %.1f tasks %.1f plan %.1f commit %.1f replay %.1f launch %.1f wait %.1f ms",
+            corpus ? "_corpus" : dout ? "_device" : "", n, tasks.size(), groups.size(), t_files, t_tasks, t_plan, t_commit, t_deliver, t_launch, t_wait);
+    if (corpus)
+      fprintf(stderr, "; K7 gathered %llu bytes in %llu pieces (%llu packets over pages) in %llu of %zu groups",
+              (unsigned long long)gathered_bytes, (unsigned long long)gathered_pieces, (unsigned long long)gathered_multi,
+              (unsigned long long)gathered_groups, groups.size());
+    fprintf(stderr, "\n");
+  }
   for (int s2 = 0; s2 < 2; s2++)
     if (ctx->bulk[s2]) vpz_batch_reset(ctx->bulk[s2]);
   return rc ? rc : total;
@@ -2089,6 +2213,119 @@ int64_t vpz_decode_excerpts_device_conv(vpz_ctx* ctx, uint32_t n_files, const ui
                                                          static_cast<float*>(dst_dev), dst_elems, dst_offsets, got, &o));
 }
 
+}  // extern "C"
+
+extern "C" {
+
+int vpz_corpus_open(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens, int copy,
+                    vpz_corpus** out) {
+  if (!ctx || !out || (n && (!datas || !lens))) return VPZ_E_ARGUMENT;
+  *out = nullptr;
+  VPZ_USE(ctx);
+  if (!ctx->pool) {
+    unsigned t = ctx->host_threads > 0 ? (unsigned)ctx->host_threads
+                                       : std::max(1u, std::min(std::thread::hardware_concurrency(), 32u));
+    ctx->pool = new (std::nothrow) ThreadPool(t);
+    if (!ctx->pool) return VPZ_E_NOMEM;
+  }
+  std::unique_ptr<vpz_corpus> c(new (std::nothrow) vpz_corpus);
+  if (!c) return VPZ_E_NOMEM;
+  c->ctx = ctx;
+  std::vector<const uint8_t*> ptrs(datas, datas + n);
+  if (copy) {
+    c->copies.resize(n);
+    for (uint32_t i = 0; i < n; i++) {
+      c->copies[i].assign(datas[i], datas[i] + lens[i]);
+      ptrs[i] = c->copies[i].data();
+    }
+  }
+  // the device images: 16-byte aligned, at least 16 zero bytes behind each (K7 reads whole aligned words)
+  c->dev_off.resize(n);
+  for (uint32_t i = 0; i < n; i++) {
+    c->dev_off[i] = c->d_bytes;
+    c->d_bytes += ((uint64_t)lens[i] + 16 + 15) & ~(uint64_t)15;
+  }
+  int rc = VPZ_OK;
+  if (c->d_bytes) {
+    c->d_img = static_cast<uint8_t*>(dev::alloc(c->d_bytes, ctx->last_error));
+    if (!c->d_img) return VPZ_E_CUDA;
+    if ((rc = dev::fill(c->d_img, 0, c->d_bytes, ctx->stream, ctx->last_error))) return rc;
+  }
+  // slices of at most "bulk_group_mib" of images: the scan's pinned staging never holds the whole corpus; each
+  // slice's images go from the scan's device copy (or, after a host scan, from the host images) into the corpus buffer
+  const uint64_t cap = ctx->bulk_group_bytes > 0 ? (uint64_t)ctx->bulk_group_bytes : (uint64_t)ctx->bulk_group_mib << 20;
+  c->files.resize(n);
+  for (uint32_t i0 = 0; i0 < n;) {
+    uint32_t i1 = i0;
+    uint64_t bytes = 0;
+    while (i1 < n && (i1 == i0 || bytes + lens[i1] <= cap)) bytes += lens[i1++];
+    std::vector<std::unique_ptr<ExcerptFile>> part(i1 - i0);
+    ScanResult sr;
+    if ((rc = open_excerpt_files(ctx, i1 - i0, ptrs.data() + i0, lens + i0, part, nullptr, &sr))) break;
+    for (uint32_t k = i0; k < i1; k++) {   // from the scan's staged images when the device scanned them
+      c->files[k] = std::move(part[k - i0]);
+      rc = sr.images ? dev::d2d(c->d_img + c->dev_off[k], sr.images + sr.files[k - i0].data_off, lens[k], ctx->stream,
+                                ctx->last_error)
+                     : dev::h2d(c->d_img + c->dev_off[k], ptrs[k], lens[k], ctx->stream, ctx->last_error);
+      if (rc) break;
+    }
+    // the copies read the scan's staged images, which the next slice's scan (on the scan stream) overwrites
+    if (rc || (rc = dev::stream_sync(ctx->stream, ctx->last_error))) break;
+    i0 = i1;
+  }
+  const std::string err = ctx->last_error;
+  const int src = dev::stream_sync(ctx->stream, ctx->last_error);   // the caller's bytes may go once open returns
+  if (rc) {
+    ctx->last_error = err;
+    return rc;
+  }
+  if (src) return src;
+  c->samples.resize(n);
+  for (uint32_t i = 0; i < n; i++) {
+    int err = 0;
+    c->samples[i] = c->files[i]->master.ls->total_granules(&err);   // cached by the open
+    if (err) return err;
+  }
+  *out = c.release();
+  return VPZ_OK;
+}
+
+void vpz_corpus_close(vpz_corpus* c) { delete c; }
+
+uint64_t vpz_corpus_device_bytes(const vpz_corpus* c) { return c ? c->d_bytes : 0; }
+
+int64_t vpz_corpus_info(const vpz_corpus* c, int32_t* channels, int32_t* sample_rate, int64_t* samples) {
+  if (!c) return VPZ_E_ARGUMENT;
+  for (size_t i = 0; i < c->files.size(); i++) {
+    const StreamDec& m = c->files[i]->master;
+    if (channels) channels[i] = m.channels();
+    if (sample_rate) sample_rate[i] = m.setup->host.id.sample_rate;
+    if (samples) samples[i] = c->samples[i];
+  }
+  return (int64_t)c->files.size();
+}
+
+int64_t vpz_corpus_excerpts_device(vpz_corpus* c, uint32_t n, const uint32_t* file_of, const int64_t* start,
+                                   const int32_t* count, int clip, const vpz_out_conv* conv, void* dst_dev,
+                                   size_t dst_elems, int64_t* dst_offsets, int32_t* got, void* stream) {
+  if (!c || (n && (!file_of || !start || !count))) return VPZ_E_ARGUMENT;
+  vpz_ctx* ctx = c->ctx;
+  VPZ_USE(ctx);
+  int rc = conv_check(ctx, conv);
+  if (rc) return rc;
+  DevOut o;
+  o.p = dst_dev;
+  o.format = conv->format;
+  o.stream = stream;
+  o.conv = conv;
+  dev::Event* ev = nullptr;
+  rc = device_output_begin(ctx, o, &ev);
+  if (rc) return device_output_end(ctx, ev, rc);
+  return device_output_end(ctx, ev, decode_excerpts_impl(ctx, (uint32_t)c->files.size(), nullptr, nullptr, n, file_of,
+                                                         start, count, clip, static_cast<float*>(dst_dev), dst_elems,
+                                                         dst_offsets, got, &o, c));
+}
+
 // Debug / tests: the page-end granule index of one container image (first logical stream), built on the device
 // (K0 + K0g; VPZ_E_UNSUPPORTED when the file does not qualify) or by the host's packet walk.  Returns the number
 // of pages, writes min(pages, cap) entries.
@@ -2119,8 +2356,9 @@ int64_t vpz_debug_page_end_granules(vpz_ctx* ctx, const uint8_t* data, size_t le
 }  // extern "C"
 
 #ifdef VPZ_EMU
-// The emulated CPU test build (tests/emu, never linked into libvpz.so) takes the K5 and K6 launchers and the
-// caller-memory hooks of the device-output calls above from here.
+// The emulated CPU test build (tests/emu, never linked into libvpz.so) takes the K5, K6 and K7 launchers and the
+// caller-memory hooks of the device-output and corpus calls above from here.
 #include "../../tests/emu/dev_emu_place.h"
 #include "../../tests/emu/dev_emu_convert.h"
+#include "../../tests/emu/dev_emu_corpus.h"
 #endif

@@ -152,6 +152,7 @@ int scan_end(vpz_ctx* ctx, int which, ScanResult* res) {
   res->files = b.h_files.p;
   res->pages = b.h_pages.p;
   res->out = b.h_out.p;
+  res->images = static_cast<const uint8_t*>(b.d_img.p);
   return VPZ_OK;
 }
 

@@ -240,6 +240,10 @@ int vpz_batch_reset(vpz_batch* b) {
   b->rec_words = b->ent_total = 0;
   b->max_channels = 1;
   b->uploaded = b->decoded = false;
+  b->gather_images = nullptr;
+  b->gather_bytes = 0;
+  b->gather_fill = nullptr;
+  b->pieces.clear();
   return VPZ_OK;
 }
 

@@ -253,6 +253,14 @@ struct VpzPlaceTile {
   uint32_t ch;              // channels
 };
 
+// ---- K7: packet bytes of a corpus call gathered from the corpus's device-resident images (k7_gather.cuh) ------
+#define VPZ_PIECE_MORE 0x80000000u             // VpzGatherPiece.len: the packet continues in the next piece
+struct VpzGatherPiece {
+  uint64_t src;             // byte offset of the piece in the corpus's images
+  uint32_t dst;             // byte offset in the batch's packet-byte area (a packet's first piece: 16-byte aligned)
+  uint32_t len;             // bytes | VPZ_PIECE_MORE when the packet's next piece follows (a packet over pages)
+};
+
 // ---- K6: rate and channel conversion into the caller's device buffer (k6_convert.cuh) ------------------------
 // Output j of an item at source rate fi and output rate fo (fi / fo = o / n in lowest terms) reads the 2 width + 2
 // source frames from floor(j o / n) - width on, weighted by phase j mod n of the rate pair's coefficient table.
