@@ -363,14 +363,17 @@ typedef struct {
  *   k in [floor(j o / n) - width, floor(j o / n) + width + 1] can be nonzero, width = ceil(6 o / (0.99 min(o, n))).
  *   ClipSamples applies to the decoded samples, before mixing and the filter; fp32 output is not clipped again,
  *   int16 clamps.  A rate pair whose coefficient table exceeds 2^22 floats fails with VPZ_E_UNSUPPORTED.
+ *   So does a stream whose one-output K6 tile needs more shared memory than the device allows per block (e.g. 8
+ *   channels to mono from 1,000,000 Hz to 1 kHz), from the size query and the call, before anything is decoded.
  * Files: sample_counts[k] = ceil(n_k fo / fi) for a converted file (n_k: vpz_decode_files' count), dst_offsets
  *   (may be NULL) the prefix sums of sample_counts * C_out (C_out = conv->channels, or the stream's when 0).  The
  *   filter sees zeros outside the file.
  * Excerpts: start / count are output-rate samples.  A converted item reads the source window k_lo =
  *   max(0, floor(start o / n) - width), k_hi = floor((start + count - 1) o / n) + width + 1 exactly as the plain call
- *   reads (k_lo, k_hi - k_lo) (width 0 at equal rates); with d samples delivered and e = k_lo + d,
- *   got = clamp(ceil(e n / o) - start, 0, count), or the negative SeekTo status.  Output samples from got on are
- *   zero.  A source window longer than the plain call takes as a count (INT32_MAX / 8 samples), or a start past
+ *   reads (k_lo, k_hi - k_lo) (width 0 at equal rates); with d samples delivered (resampled: those before the
+ *   stream's TotalSamples; the filter sees zeros from there on, as in the files call, although a reader that seeks
+ *   into the last packet delivers it untrimmed) and e = k_lo + d, got = clamp(ceil(e n / o) - start, 0, count), or the negative SeekTo
+ *   status.  Output samples from got on are zero.  A source window longer than the plain call takes as a count (INT32_MAX / 8 samples), or a start past
  *   2^40 samples, fails with VPZ_E_ARGUMENT.
  * channels = 2 with a source of more than 2 channels fails with VPZ_E_UNSUPPORTED before anything is decoded. */
 int64_t vpz_decode_files_device_conv(vpz_ctx* ctx, uint32_t n, const uint8_t* const* datas, const size_t* lens,

@@ -10,10 +10,16 @@
 namespace vpz {
 namespace dev {
 
-// K6: the unmodified kernel body, two emulated CTAs of 64 threads grid-striding over the tiles
-int launch_k6(const K6Params& p, Stream*, std::string&) {
+// K6: the unmodified kernel body, two emulated CTAs of 64 threads grid-striding over the tiles; the device's
+// shared-memory limit applies as on the GPU
+int launch_k6(const K6Params& p, Stream*, std::string& err) {
   if (p.n_tiles == 0) return VPZ_OK;
-  emu::launch(2, 64, (size_t)p.smem_floats * 4, [&] {
+  const size_t smem = (size_t)p.smem_floats * 4;
+  if (smem > max_smem_per_block()) {
+    err = "vpz_k6_convert: a tile needs " + std::to_string(smem) + " bytes of shared memory";
+    return VPZ_E_UNSUPPORTED;
+  }
+  emu::launch(2, 64, smem, [&] {
     float* sm = static_cast<float*>(emu::t_block->smem);
     if (p.out16) {
       if (p.planar) k6_cta<true, true>(p, sm); else k6_cta<true, false>(p, sm);

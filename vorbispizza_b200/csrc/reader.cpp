@@ -1098,6 +1098,14 @@ int conv_plan(vpz_ctx* ctx, const vpz_out_conv& cv, int fi, int C, bool build, I
   while (m > 1 && span(m) > budget) m--;
   ic->m = (uint32_t)m;
   ic->smem_floats = (uint32_t)(span(m) * per_frame);
+  // a one-output tile that still does not fit (thousands of taps times many staged channels) fails here, before
+  // anything is decoded, and so does the size query; launch_k6 keeps the same check as a backstop
+  if ((size_t)ic->smem_floats * 4 > dev::max_smem_per_block()) {
+    ctx->last_error = "conversion: a K6 tile of " + std::to_string(fi) + " -> " + std::to_string(fo) + " Hz from " +
+                      std::to_string(C) + " channels needs " + std::to_string((size_t)ic->smem_floats * 4) +
+                      " bytes of shared memory, more than the device's " + std::to_string(dev::max_smem_per_block());
+    return VPZ_E_UNSUPPORTED;
+  }
   return VPZ_OK;
 }
 
@@ -1716,11 +1724,18 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
   const int32_t* ocount = count;
   std::vector<int64_t> xstart;
   std::vector<int32_t> xcount;
+  // the filter of a resampled excerpt sees its file as the files call decodes it: TotalSamples samples, zeros after
+  // them.  (A reader that seeks into the last packet delivers that packet untrimmed; the plain call and the
+  // equal-rate mix keep those samples, the filter must not see them.)
+  std::vector<int64_t> fend(cv ? n_files : 0, INT64_MAX);
   if (cv) {
     for (uint32_t f = 0; f < n_files; f++) {
       const StreamDec& m = files[f]->master;
       int rc = conv_plan(ctx, *cv, m.setup->host.id.sample_rate, m.channels(), dst != nullptr, &fconv[f]);
       if (rc) return rc;
+      int err = 0;
+      const int64_t total = fconv[f].filter ? m.ls->total_granules(&err) : -1;   // (cached by open_excerpt_files)
+      if (!err && total >= 0) fend[f] = total;
     }
     xstart.resize(n);
     xcount.resize(n);
@@ -2038,11 +2053,16 @@ static int64_t decode_excerpts_impl(vpz_ctx* ctx, uint32_t n_files, const uint8_
         }
         d->seg_sink = nullptr;
         if (got) got[i] = src ? src : have;
-        if (conv_on) {   // the window's segments into the scratch, then K6
+        if (conv_on) {   // the window's segments (resampled: those inside the file) into the scratch, then K6
           const uint64_t item = (uint64_t)(dst_offsets[i] - g.base);
-          for (size_t sg = mark; sg < segs.size(); sg++)
-            append_tiles(task_xtiles[k], segs[sg].src, xoff[i], count[i], (segs[sg].dst - item) / C, segs[sg].n / C, C);
-          conv_item(k, i, src ? 0 : have, src);
+          const int inside = (int)std::min<int64_t>(have, std::max<int64_t>(0, fend[t.file] - start[i]));
+          for (size_t sg = mark; sg < segs.size(); sg++) {
+            const uint64_t first = (segs[sg].dst - item) / C;
+            if (first < (uint64_t)inside)
+              append_tiles(task_xtiles[k], segs[sg].src, xoff[i], count[i], first,
+                           std::min<uint64_t>(segs[sg].n / C, (uint64_t)inside - first), C);
+          }
+          conv_item(k, i, src ? 0 : inside, src);
         } else if (dout) {   // the segments (samples [0, have)), then zeros up to count
           const uint64_t item = (uint64_t)(dst_offsets[i] - g.base);
           for (size_t sg = mark; sg < segs.size(); sg++)
